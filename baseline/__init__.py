@@ -1,8 +1,8 @@
 """The reference itself, for the drop-in test and the Python CPU baseline of bench.py.
 
-`baseline/_ref/` is a git-ignored COPY of /root/reference/src made by `__graft_entry__.build()` in the build container
-(the reference is a plain source tree: there is nothing to pip-install).  It ships to the GPU box with the snapshot;
-nothing here is imported by the product (marl_uavs_targets_tracking_b200/) -- only tests/ and bench.py use it, and both
+`baseline/_ref/` is a git-ignored COPY of the reference's `src/` made by `__graft_entry__.build()` when
+UAVSIM_REFERENCE_SRC names a checkout of it (the reference is a plain source tree: there is nothing to pip-install).
+Nothing here is imported by the product (marl_uavs_targets_tracking_b200/) -- only tests/ and bench.py use it, and both
 skip cleanly when the copy is absent.
 """
 import os
@@ -14,9 +14,10 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 REF_DIR = os.path.join(HERE, "_ref", "src")
 
 
-def sync_reference(src="/root/reference/src"):
-    """Copy the reference's src/ into baseline/_ref/src (build container only).  Returns the path or None."""
-    if not os.path.isdir(src):
+def sync_reference(src=None):
+    """Copy the reference's src/ (default: $UAVSIM_REFERENCE_SRC) into baseline/_ref/src.  Returns the path or None."""
+    src = src or os.environ.get("UAVSIM_REFERENCE_SRC")
+    if not src or not os.path.isdir(src):
         return REF_DIR if os.path.isdir(REF_DIR) else None
     if os.path.isdir(REF_DIR):
         shutil.rmtree(REF_DIR)
@@ -32,7 +33,7 @@ def import_reference():
     """Import the UNMODIFIED reference modules from baseline/_ref/src.  src/train.py pulls matplotlib / imageio in
     through utils.draw_util (absent in this image): that one module is stubbed (SURVEY.md section 8c), nothing else."""
     if not available():
-        raise ImportError("baseline/_ref/src is missing: run __graft_entry__.build() where /root/reference exists")
+        raise ImportError("baseline/_ref/src is missing: run __graft_entry__.build() with UAVSIM_REFERENCE_SRC set")
     sys.dont_write_bytecode = True
     if REF_DIR not in sys.path:
         sys.path.insert(0, REF_DIR)

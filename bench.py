@@ -17,6 +17,12 @@ e2e       = same metric through BatchedEnvironment.step_host (the C-ABI call wit
 roofline  = algorithmic bytes per launch (SURVEY.md section 8d: 124 n + 48 m + 4 per env-step) / mean launch time
             against the measured HBM copy bandwidth in MEASURED_PEAKS.json.
 cpu_baseline = the CPU oracle (C port of the reference loop, oracle/) on a bounded sample, all host threads.
+             cpu_baseline.python_reference times the reference's own Python step; it needs the copy of the
+             reference that __graft_entry__.build() makes from $UAVSIM_REFERENCE_SRC and is null without it.
+
+--dump-outputs DIR writes what the last timed step returned (observations, reward planes, covered counts; a fixed
+sample of environments when the workload is large) as .npy files.  The inputs depend only on the arguments, so two
+builds of the project can be compared output for output.
 """
 import argparse
 import json
@@ -170,6 +176,26 @@ class ClockSampler:
                 "power_w_max": max(pw) if pw else None, "samples": len(sm), "window": window, "reasons": sorted(reasons)}
 
 
+DUMP_BYTES = 32 << 20  # --dump-outputs: above this, a seeded sample of the environments is written
+
+
+def dump_outputs(out_dir, obs, rew4, covered):
+    """Write one step's outputs as returned by step_device -- obs [E,n,12] and rew4 [4,E,n] float32, covered [E] (as
+    float64) -- to out_dir/<name>.npy.  When all E environments exceed DUMP_BYTES, a fixed seeded sample of them is
+    written in ascending order; env_index.npy (float64) says which environments the rows are."""
+    import numpy as np
+    import torch
+    E, n = obs.shape[0], obs.shape[1]
+    k = min(E, DUMP_BYTES // ((12 + 4) * n * 4 + 2 * 8))
+    idx = np.arange(E) if k == E else np.sort(np.random.RandomState(0).choice(E, k, replace=False))
+    sel = torch.from_numpy(idx).to(obs.device)
+    arrays = {"obs": obs.index_select(0, sel).float(), "rew4": rew4.index_select(1, sel).float(),
+              "covered": covered.index_select(0, sel).double(), "env_index": torch.from_numpy(idx).double()}
+    os.makedirs(out_dir, exist_ok=True)
+    for name, t in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), t.cpu().numpy())
+
+
 def make_pmi(torch, hidden=128):
     from marl_uavs_targets_tracking_b200 import PMINetwork
     torch.manual_seed(42)
@@ -301,7 +327,7 @@ def measure_workload(torch, dist, env_cls, args, name, rank, world, device, step
         if i % EPISODE == 0 and i > 0:
             env.reset(cfg)
         env.bind_actions(bank[i % NB])
-        env.step_device(cfg, pmi)
+        return env.step_device(cfg, pmi)
 
     def barrier():
         torch.cuda.synchronize(device)
@@ -318,7 +344,7 @@ def measure_workload(torch, dist, env_cls, args, name, rank, world, device, step
     ev0.record(torch.cuda.current_stream(device))
     marks = []
     for i in range(steps):
-        one_step(warmup + i)
+        last = one_step(warmup + i)
         if args.trace_every and (i + 1) % args.trace_every == 0:
             e = torch.cuda.Event(enable_timing=True)
             e.record(torch.cuda.current_stream(device))
@@ -326,6 +352,8 @@ def measure_workload(torch, dist, env_cls, args, name, rank, world, device, step
     ev1.record(torch.cuda.current_stream(device))
     barrier()
     clocks = sampler.stop(t_begin, time.time())
+    if args.dump_outputs and name == args.workload and rank == 0:
+        dump_outputs(args.dump_outputs, *last)  # before the legs below overwrite the output buffers
     ms = ev0.elapsed_time(ev1)
     launches = env.launch_count() - l0
     trace = None
@@ -501,7 +529,13 @@ def main():
     ap.add_argument("--trace-every", type=int, default=0, help="also report ms/step per window of this many steps")
     ap.add_argument("--no-extras", action="store_true", help="skip the secondary workloads and the CPU baseline")
     ap.add_argument("--step-path", type=int, default=0, help="step kernel: 0 default, 1 generic, 2 per-UAV walks (64x64), 3 all-pairs tiles (64x64), 4 small-swarm")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the last timed step's outputs (rank 0's environments) "
+                    "as DIR/<name>.npy: obs, rew4, covered, env_index")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "native":
+        ap.error("--dump-outputs writes the outputs of the native step")
     args.warmup = max(args.warmup, 3) if args.impl == "native" else args.warmup
 
     rank = int(os.environ.get("RANK", "0"))

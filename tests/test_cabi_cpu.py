@@ -29,10 +29,10 @@ def test_every_declared_symbol_is_exported_and_bound():
     assert declared == set(_cabi.SYMBOLS), "ctypes table and header disagree: %s" % (declared ^ set(_cabi.SYMBOLS))
 
 
-def test_struct_layouts_match_the_header():
+def test_struct_layouts_match_the_header(tmp_path):
     """sizeof() seen by the C compiler == ctypes layout (catches field drift)."""
     src = '#include <stdio.h>\n#include "uavsim.h"\nint main(){printf("%zu %zu %zu\\n", sizeof(UavSimParams), sizeof(UavSimBuffers), sizeof(UavSimPmiWeights));return 0;}'
-    exe = "/tmp/uavsim_sizeof"
+    exe = str(tmp_path / "uavsim_sizeof")
     subprocess.run(["gcc", "-x", "c", "-", "-I", os.path.join(ROOT, "include"), "-o", exe], input=src.encode(), check=True)
     a, b, c = map(int, subprocess.check_output([exe]).split())
     assert (a, b, c) == (C.sizeof(_cabi.UavSimParams), C.sizeof(_cabi.UavSimBuffers), C.sizeof(_cabi.UavSimPmiWeights))
@@ -59,7 +59,7 @@ def test_argument_errors_are_reported():
     assert b"NULL" in lib.uavsim_last_error()
 
 
-def test_philox_host_build_matches_numpy_reference():
+def test_philox_host_build_matches_numpy_reference(tmp_path):
     """csrc/philox.cuh compiled for the host equals tests/philox_ref.py and the Random123 known answers."""
     import numpy as np
     from philox_ref import philox4x32_10, u53
@@ -70,7 +70,7 @@ int main(){ unsigned c[3][4]={{0,0,0,0},{0xffffffffu,0xffffffffu,0xffffffffu,0xf
  unsigned long long k[3]={0ull,0xffffffffffffffffull,0x299f31d0a4093822ull};
  for(int i=0;i<3;i++){Philox4 r=philox4x32_10(c[i][0],c[i][1],c[i][2],c[i][3],k[i]); printf("%08x %08x %08x %08x %.17g\n",r.v[0],r.v[1],r.v[2],r.v[3],philox_u53(r.v[0],r.v[1]));}
  return 0;}'''
-    exe = "/tmp/uavsim_philox"
+    exe = str(tmp_path / "uavsim_philox")
     subprocess.run(["g++", "-x", "c++", "-", "-I", os.path.join(ROOT, "marl_uavs_targets_tracking_b200", "csrc"), "-o", exe], input=src.encode(), check=True)
     lines = subprocess.check_output([exe]).decode().strip().split("\n")
     kat = ["6627e8d5 e169c58d bc57ac4c 9b00dbd8", "408f276d 41c83b0e a20bc7c6 6d5451fd", "d16cfe09 94fdcceb 5001e420 24126ea1"]

@@ -10,6 +10,10 @@
 for all three methods with the shipped YAML files.  The recorded transitions are then replayed step by step in the
 reference's own `Environment` (same initial state, same actions): next states, the four reward lists and the covered
 count must agree within the contract (1e-5; integer count exact), so the numbers the learner saw are the reference's.
+
+Without that copy, the same comparison runs against episodes recorded from the reference's own `Environment.step`
+(tests/golden/d10_*.npz, made by tests/golden/make_golden.py): the single-environment drop-in replays them through the
+reference-shaped API and must reproduce every step.
 """
 import random
 
@@ -17,17 +21,20 @@ import numpy as np
 import pytest
 import torch
 
-from gpu_util import max_scaled_err
+from conftest import load_golden
+from gpu_util import STATE, golden_config, golden_pmi_module, max_scaled_err
 
 pytestmark = pytest.mark.gpu
 
 TOL = 1e-5
+REWARDS = (("rewards", "rewards"), ("target_tracking_reward", "tt"), ("boundary_punishment", "bp"),
+           ("duplicate_tracking_punishment", "dup"))
 
 
 def _reference():
     import baseline
     if not baseline.available():
-        pytest.skip("baseline/_ref/src absent (build() copies it where /root/reference exists)")
+        pytest.skip("baseline/_ref/src absent (build() copies it from $UAVSIM_REFERENCE_SRC)")
     return baseline, baseline.import_reference()
 
 
@@ -95,4 +102,49 @@ def test_reference_operate_epoch_drives_the_cuda_environment(method):
     ref_returns = sums / (T * n)
     assert np.allclose([ret, tt_ret, bp_ret, dup_ret], ref_returns, rtol=0, atol=TOL)
     assert avg_cov == pytest.approx(np.mean(covs)) and max_cov == np.max(covs)
+    env.close()
+
+
+@pytest.mark.parametrize("seed", [42, 7])
+@pytest.mark.parametrize("method", ["MAAC", "MAAC-G", "MAAC-R"])
+def test_reference_shaped_environment_replays_the_reference_recordings(method, seed):
+    """The single-environment drop-in, built and configured the way src/main.py does it with the shipped YAML values,
+    replays a 200-step episode recorded from the reference's own `Environment.step` (same initial state, same actions,
+    for MAAC-R the recorded PMINetwork state_dict).  Next states, the four reward lists, the covered count, the
+    `uav_list` views, the position / coverage traces and the returns operate_epoch reports must be the reference's."""
+    from marl_uavs_targets_tracking_b200 import Environment, default_config
+    g = load_golden("d10_%s_s%d" % ({"MAAC": "self", "MAAC-G": "mean", "MAAC-R": "pmi"}[method], seed))
+    cfg = default_config(method)
+    rec = golden_config(g)
+    assert all(cfg[k] == rec[k] for k in ("cooperative", "environment", "uav", "target"))  # the recorded scenario
+    e = cfg["environment"]
+    n, T = e["n_uav"], int(g["params_i"][3])
+    pmi = golden_pmi_module(g) if method == "MAAC-R" else None
+
+    env = Environment(n_uav=n, m_targets=e["m_targets"], x_max=e["x_max"], y_max=e["y_max"], na=e["na"])
+    env.reset(cfg)
+    env.set_state(cfg, *(np.asarray(g[k + "0"])[None] for k in STATE))
+    assert max_scaled_err(np.stack([u.get_local_state() for u in env.uav_list]), g["obs0"]) <= TOL
+    worst, pos = 0.0, 0.0
+    sums, ref_sums = np.zeros(4), np.zeros(4)
+    for t in range(T):
+        ns, rew, cov = env.step(cfg, pmi, [int(a) for a in g["actions"][t]])
+        assert isinstance(ns, list) and len(ns) == n and all(s.shape == (12,) and s.dtype == np.float64 for s in ns)
+        assert isinstance(cov, int) and cov == int(g["covered"][t]), (t, "covered")
+        worst = max(worst, max_scaled_err(np.stack(ns), g["obs"][t]))
+        for q, (key, gk) in enumerate(REWARDS):
+            assert len(rew[key]) == n
+            worst = max(worst, max_scaled_err(np.asarray(rew[key]), g[gk][t]))
+            sums[q] += sum(rew[key])
+            ref_sums[q] += g[gk][t].sum()
+        np.testing.assert_array_equal(np.stack(ns), np.stack([u.get_local_state() for u in env.uav_list]))
+        for attr, gk in (("x", "ux"), ("y", "uy"), ("h", "uh")):
+            pos = max(pos, max_scaled_err([getattr(u, attr) for u in env.uav_list], g[gk][t]))
+        assert [u.a for u in env.uav_list] == [int(a) for a in g["actions"][t]]
+    print(method, seed, "worst %.1e, positions %.1e" % (worst, pos))
+    assert worst <= TOL and pos <= 1e-9
+    assert env.covered_target_num == [int(c) for c in g["covered"]]
+    for key, gk in (("all_uav_xs", "ux"), ("all_uav_ys", "uy"), ("all_target_xs", "tx"), ("all_target_ys", "ty")):
+        assert max_scaled_err(np.asarray(env.position[key]), g[gk]) <= 1e-9, key
+    assert np.allclose(sums / (T * n), ref_sums / (T * n), rtol=0, atol=TOL)
     env.close()
