@@ -164,14 +164,17 @@ int uavsim_set_pmi_weights(uavsim_t *h, const UavSimPmiWeights *w, void *stream)
  * for tests and A/B timing. */
 int uavsim_set_step_path(uavsim_t *h, int path);
 
-/* Which kernel evaluates the PMI MLP: 0 = automatic (tensor cores when hidden is 64 or 128 and the neighbour lists fit),
- * 1 = fp32 CUDA cores, 2 = tcgen05 tensor cores with split fp16 hi + lo operands (error if unsupported). */
+/* Which kernel evaluates the PMI MLP: 0 = automatic (tensor cores when hidden is 64 or 128, the neighbour lists fit and
+ * the fc1 weights fit fp16 after the per-unit rebalancing of uavsim_set_pmi_weights), 1 = fp32 CUDA cores, 2 = tcgen05
+ * tensor cores with split fp16 hi + lo operands (error if unsupported, also when weights uploaded later do not fit). */
 int uavsim_set_pmi_path(uavsim_t *h, int path);
 
 /* Episode statistics accumulated by uavsim_step since the last reset (src/train.py:181-192):
  * out[0..3] = sums of rewards / tracking / boundary / duplicate over env-steps and UAVs,
  * out[4] = sum of covered_targets over env-steps, out[5] = max covered_targets,
- * out[6] = env-steps accumulated, out[7] = 0.  Synchronises `stream`.  The reward sums of the step kernels are
+ * out[6] = env-steps accumulated, out[7] = pair rows the tensor-core PMI kernel evaluated with inputs beyond the range its
+ * fp16 activations hold for the uploaded weights (their logits saturate; 0 in any run the tensor path serves exactly,
+ * DESIGN.md section 3.2; the CUDA-core kernel has no such limit and never counts).  Synchronises `stream`.  The reward sums of the step kernels are
  * accumulated as integer counts of 2^-22 per (environment, UAV, step) -- exact in any order, so the totals are
  * bit-reproducible although CTAs draw their environments from a counter; resolution 2.4e-7 per value. */
 int uavsim_episode_stats(uavsim_t *h, double out[8], void *stream);

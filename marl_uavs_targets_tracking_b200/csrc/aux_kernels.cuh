@@ -83,19 +83,22 @@ __global__ void uavsim_stats_reduce_kernel(const double *__restrict__ partial, i
   }
   {  // third region: the fast step kernel's reward sums as 64-bit counts of 2^-22 (exact in any order)
     const long long *fx = reinterpret_cast<const long long *>(partial + (size_t)2 * slots * STAT_W);
-    long long c[4] = {0, 0, 0, 0};
+    // (field 4: pair rows the tensor PMI kernel found beyond its fp16 range, a plain count -> out[7])
+    long long c[5] = {0, 0, 0, 0, 0};
     for (int s = threadIdx.x; s < slots; s += 256)
-      for (int k = 0; k < 4; k++) c[k] += fx[(size_t)s * STAT_W + k];
-    __shared__ long long shc[256][4];
-    for (int k = 0; k < 4; k++) shc[threadIdx.x][k] = c[k];
+      for (int k = 0; k < 5; k++) c[k] += fx[(size_t)s * STAT_W + k];
+    __shared__ long long shc[256][5];
+    for (int k = 0; k < 5; k++) shc[threadIdx.x][k] = c[k];
     __syncthreads();
     for (int w = 128; w > 0; w >>= 1) {
       if ((int)threadIdx.x < w)
-        for (int k = 0; k < 4; k++) shc[threadIdx.x][k] += shc[threadIdx.x + w][k];
+        for (int k = 0; k < 5; k++) shc[threadIdx.x][k] += shc[threadIdx.x + w][k];
       __syncthreads();
     }
-    if (threadIdx.x == 0)
+    if (threadIdx.x == 0) {
       for (int k = 0; k < 4; k++) a[k] += (double)shc[0][k] * (1.0 / 4194304.0);
+      a[7] = (double)shc[0][4];
+    }
   }
   for (int k = 0; k < STAT_W; k++) sh[threadIdx.x][k] = a[k];
   __syncthreads();
@@ -104,6 +107,7 @@ __global__ void uavsim_stats_reduce_kernel(const double *__restrict__ partial, i
       for (int k = 0; k < 5; k++) sh[threadIdx.x][k] += sh[threadIdx.x + w][k];
       sh[threadIdx.x][5] = fmax(sh[threadIdx.x][5], sh[threadIdx.x + w][5]);
       sh[threadIdx.x][6] += sh[threadIdx.x + w][6];
+      sh[threadIdx.x][7] += sh[threadIdx.x + w][7];
     }
     __syncthreads();
   }

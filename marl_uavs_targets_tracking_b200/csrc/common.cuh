@@ -129,10 +129,12 @@ struct uavsim {
   int pmi_g, pmi_pmax, pmi_tm, pmi_grid_max;
   // tensor-core path (H = 128): fc1 pre-split into UMMA tiles
   bool has_tc;
+  bool tc_range;  // the rebalanced weights fit the tensor path's fp16 operands (false: hidden 64 / 128 served by CUDA cores)
   bool has_cc;   // the fp32 CUDA-core PMI kernel fits this shape (its pair buffer is 8 192 rows; n > 91 needs the tensor path)
   int pmi_path;        // 0 auto, 1 CUDA cores, 2 tensor cores
   float *d_tc_tiles;   // [12][2][128*32]
   int tc_g;
+  float tc_x_safe;     // largest |input| of a pair row the tensor path's fp16 activations hold (rows beyond are counted)
   size_t smem_pmi;
   // host-buffer pipeline
   cudaStream_t s_in, s_comp, s_out;

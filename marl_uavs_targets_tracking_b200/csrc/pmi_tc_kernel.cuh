@@ -77,6 +77,13 @@
 #error "the TF32 variant keeps two producer threads per row: build it with -DTC_F16=0 -DTC_PARTS=2"
 #endif
 #define TC_STAGE_BYTES (2 * TC_A_BYTES)  // B_hi + B_lo
+// Per-unit rebalancing of the uploaded weights (uavsim_set_pmi_weights): row u of layer 0 is scaled by a power of two so
+// that max(b0_u, 0) + PMI_X_NOM * sum_k |w0_uk| lies in [2^PMI_BAL_T, 2^(PMI_BAL_T+1)), column u of fc1 by the inverse.  This puts
+// the fp16 activations of inputs up to PMI_X_NOM below 2^(PMI_BAL_T+1) and leaves fc1 times TC_WSCALE room up to 65504:
+// with T = 8 and X = 16 the tensor path holds pair-row inputs up to ~2 000 and a folded fc1 weight up to ~1 000 on the
+// units of an untrained network (DESIGN.md section 3.2).
+#define PMI_BAL_T 8
+#define PMI_X_NOM 16.0
 #define TC_ACOL0 256u        // first TMEM column of the A ring
 #define TC_AMAX 512          // UAVs per environment group
 #define TC_PMAX 16384        // neighbour pairs per environment group (logits stay in shared memory until the softmax)
@@ -178,7 +185,8 @@ __device__ __forceinline__ void tmem_st4(uint32_t taddr, const uint32_t *u) {
 // acc = {row 0, row 1} of unit u, acc2 = the same of unit u'.  hi is the value truncated to 11 significant bits (one AND), so
 // v - hi is exact, has the sign of v, and both conversions are exact up to the final rounding of lo to 11 bits.  The ReLU
 // rides on the conversions (.relu: a negative v gives hi = lo = 0); .satfinite keeps an activation beyond fp16's range finite
-// (it does not occur with weights that produce finite rewards).  Outputs: packed {u, u'} per row (lower K index in the low half).
+// (an activation that large comes from a pair row whose inputs exceed PmiTcDev::x_safe; the kernel counts those rows in
+// the statistics, pmi_rows_out_of_range, instead of failing).  Outputs: packed {u, u'} per row (lower K index in the low half).
 __device__ __forceinline__ void tc_relu_split(uint64_t acc, uint64_t acc2, uint32_t &hi_r0, uint32_t &lo_r0, uint32_t &hi_r1, uint32_t &lo_r1) {
   const uint64_t m = 0xffffe000ffffe000ull;
   const uint64_t h = acc & m, h2 = acc2 & m;
@@ -231,6 +239,7 @@ struct PmiTcDev {
   const float *w0, *b0, *b1, *w2;  // [384*5] [384] [128] [128] folded fp32
   const float *w1_tiles;           // [24][2][128 x 16] fc1 pre-split (hi | lo) in the UMMA layout
   float b2;
+  float x_safe;                    // largest max_k |x_k| of a pair row whose layer-0 activations fit fp16 (host-computed)
 };
 
 template <int H>   // hidden size of the PMI network: 128 (src/configs/*.yaml) or 64 (the default of PMINetwork's constructor)
@@ -299,6 +308,7 @@ uavsim_pmi_tc_kernel(const KParams P, const UavSimBuffers B, const PmiTcDev W, i
   // draws one group ahead; every role reads the index behind the barrier at the loop top.  The reward sum is a
   // fixed-point count for the same reason as in the step kernels (common.cuh: sf_fx).
   long long fx_r = 0;
+  int oor = 0;  // pair rows beyond W.x_safe built by this producer (counted by the threads of unit part 0 only)
   long long *const s_next = reinterpret_cast<long long *>(smem + TcSmem::bar + 112);  // (mbarriers end at +112 at most, the tensor-memory pointer sits at +120)
   long long drawn = 0;
   if (tid == 0 && (int64_t)blockIdx.x < ngroups) drawn = (long long)gridDim.x + (long long)atomicAdd(P.fast_ctr, 1);
@@ -418,8 +428,10 @@ uavsim_pmi_tc_kernel(const KParams P, const UavSimBuffers B, const PmiTcDev W, i
             if (k >= c0) { k -= c0; w = s_nbr[2 * a + 1]; base += 64; }
             for (int q = 0; q < k; q++) w &= w - 1;
             const int b = base + __ffsll((long long)w) - 1;
+            float mx = 0.f;
 #pragma unroll
-            for (int q = 0; q < 12; q++) x[q] = s_obs[a * 12 + q] * s_obs[b * 12 + q];
+            for (int q = 0; q < 12; q++) { x[q] = s_obs[a * 12 + q] * s_obs[b * 12 + q]; mx = fmaxf(mx, fabsf(x[q])); }
+            oor += (half == 0 && mx > W.x_safe) ? 1 : 0;
           } else {
 #pragma unroll
             for (int q = 0; q < 12; q++) x[q] = 0.f;
@@ -596,6 +608,11 @@ uavsim_pmi_tc_kernel(const KParams P, const UavSimBuffers B, const PmiTcDev W, i
     if (atomicAdd(P.fast_ctr + 1, 1) == (int)gridDim.x - 1) { P.fast_ctr[0] = 0; P.fast_ctr[1] = 0; __threadfence(); }
   }
   // (stats_partial is the PMI region of the statistics array; the fixed-point region follows it)
-  block_stats_commit_fx(reinterpret_cast<long long *>(s_red),
-                        reinterpret_cast<long long *>(stats_partial + (size_t)P.stat_slots * STAT_W) + (size_t)blockIdx.x * STAT_W, fx_r, 0, 0, 0);
+  long long *const slot = reinterpret_cast<long long *>(stats_partial + (size_t)P.stat_slots * STAT_W) + (size_t)blockIdx.x * STAT_W;
+  block_stats_commit_fx(reinterpret_cast<long long *>(s_red), slot, fx_r, 0, 0, 0);
+  // field 4: pair rows out of the fp16 range (integer, so the order of the warps' additions does not matter)
+  if (producer) {
+    const int c = __reduce_add_sync(0xffffffffu, oor);
+    if (lane == 0 && c) atomicAdd(reinterpret_cast<unsigned long long *>(slot + 4), (unsigned long long)c);
+  }
 }

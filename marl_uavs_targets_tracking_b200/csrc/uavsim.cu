@@ -10,6 +10,8 @@
 // SURVEY.md section 7), compiled with -fmad=false so the parity-critical expressions keep the
 // reference's evaluation order.  Range tests compare squared distances against the exact squared
 // threshold computed on the host (largest double s with sqrt(s) <= thr), and take sqrt only on hits.
+#include <cfloat>
+#include <cmath>
 #include <mutex>
 #include <vector>
 
@@ -484,16 +486,23 @@ static float host_tf32_rna(float v) {
 }
 #endif
 
-static bool pmi_use_tensor(const uavsim_t *h) {
-  if (!h->has_tc || h->pmi_path == 1) return false;
+// the tensor path can serve this shape and these weights (whatever uavsim_set_pmi_path asked for)
+static bool pmi_tensor_available(const uavsim_t *h) {
   const int n = h->kp.n;
-  return n * (n - 1) <= TC_PMAX && n <= TC_AMAX;
+  return h->has_tc && n * (n - 1) <= TC_PMAX && n <= TC_AMAX;
+}
+static bool pmi_use_tensor(const uavsim_t *h) { return h->pmi_path != 1 && pmi_tensor_available(h); }
+static const char *pmi_tensor_why_not(const uavsim_t *h) {
+  if (h->has_pmi && (h->pmi.H == 64 || h->pmi.H == 128) && !h->tc_range)
+    return "these weights exceed the fp16 range of its operands after the per-unit rebalancing (the CUDA-core kernel serves them)";
+  return "the tensor-core path needs hidden = 64 or 128 and n_uav*(n_uav-1) <= 16384";
 }
 
 static int pmi_tc_launch(uavsim_t *h, int64_t e0, int64_t cnt, double coop, cudaStream_t st) {
   PmiTcDev W;
   W.w0 = h->pmi.w0; W.b0 = h->pmi.b0; W.b1 = h->pmi.b1; W.w2 = h->pmi.w2; W.b2 = h->pmi.b2;
   W.w1_tiles = h->d_tc_tiles;
+  W.x_safe = h->tc_x_safe;
   // Group size: the largest that fits (tc_g) fixes the number of waves over the one-CTA-per-SM grid; within that number
   // of waves the groups are made equal, so that every CTA gets the same count (16 384 environments of 10 UAVs: 51 per
   // group would be 322 groups = 2.2 per CTA, i.e. three for some and two for most; 37 per group is 443 = three for all).
@@ -521,6 +530,10 @@ static int pmi_tc_launch(uavsim_t *h, int64_t e0, int64_t cnt, double coop, cuda
 
 static int pmi_launch(uavsim_t *h, int64_t e0, int64_t cnt, double coop, cudaStream_t st, bool configure_only) {
   if (!configure_only && pmi_use_tensor(h)) return pmi_tc_launch(h, e0, cnt, coop, st);
+  if (!configure_only && h->pmi_path == 2) {  // (weights uploaded after the path was chosen)
+    SET_ERR("PMI mode: tensor-core path selected (uavsim_set_pmi_path 2) but unavailable: %s", pmi_tensor_why_not(h));
+    return UAVSIM_ERR_UNSUPPORTED;
+  }
   if (!configure_only && !h->has_cc) {
     SET_ERR("PMI mode: n_uav=%d is too large for the CUDA-core PMI kernel and the tensor path is %s", h->kp.n,
             h->pmi_path == 1 ? "switched off (uavsim_set_pmi_path 1)" : "unavailable (hidden is neither 64 nor 128)");
@@ -538,8 +551,8 @@ static int pmi_launch(uavsim_t *h, int64_t e0, int64_t cnt, double coop, cudaStr
 
 extern "C" int uavsim_set_pmi_path(uavsim_t *h, int path) {
   if (!h || path < 0 || path > 2) { SET_ERR("uavsim_set_pmi_path: bad argument"); return UAVSIM_ERR_ARG; }
-  if (path == 2 && h->has_pmi && !pmi_use_tensor(h) && !(h->has_tc && h->pmi_path == 1)) {
-    SET_ERR("uavsim_set_pmi_path: the tensor-core path needs hidden = 64 or 128 and n_uav*(n_uav-1) <= %d", TC_PMAX);
+  if (path == 2 && h->has_pmi && !pmi_tensor_available(h)) {
+    SET_ERR("uavsim_set_pmi_path: %s", pmi_tensor_why_not(h));
     return UAVSIM_ERR_UNSUPPORTED;
   }
   h->pmi_path = path;
@@ -562,7 +575,8 @@ extern "C" int uavsim_set_pmi_weights(uavsim_t *h, const UavSimPmiWeights *w, vo
   cudaStream_t st = (cudaStream_t)stream;
   const size_t n_w0 = (size_t)3 * H * 5, n_b0 = 3 * H, n_w1 = (size_t)H * 3 * H, n_b1 = H, n_w2 = H;
   const size_t total = n_w0 + n_b0 + n_w1 + n_b1 + n_w2;
-  float *blob = (float *)malloc(total * sizeof(float));
+  std::vector<float> blob_v(total);  // (kept until the tensor tiles are built from it)
+  float *blob = blob_v.data();
   float *q = blob;
   memcpy(q, w->w0, n_w0 * 4); q += n_w0;
   memcpy(q, w->b0, n_b0 * 4); q += n_b0;
@@ -571,11 +585,67 @@ extern "C" int uavsim_set_pmi_weights(uavsim_t *h, const UavSimPmiWeights *w, vo
   q += n_w1;
   memcpy(q, w->b1, n_b1 * 4); q += n_b1;
   memcpy(q, w->w2, n_w2 * 4);
+  // Per-unit rebalancing (DESIGN.md section 3.2): ReLU is positively homogeneous, so row u of layer 0 (w0, b0) times
+  // 2^s_u and column u of fc1 times 2^-s_u is the same function; with powers of two the fp32 arithmetic of the CUDA-core
+  // kernel gives bit-identical results.  s_u brings max(b0_u, 0) + PMI_X_NOM * sum_k |w0_uk| (the activation bound for
+  // inputs up to PMI_X_NOM: a negative pre-activation is 0 after the ReLU) to [2^PMI_BAL_T, 2^(PMI_BAL_T+1)), which
+  // puts the tensor path's fp16 activations and fc1 halves at the same magnitudes whatever scale the BatchNorm folding
+  // gave the unit; it is raised where the fc1 column would otherwise leave fp16's range after the TC_WSCALE pre-scale
+  // (that unit's activations then take a smaller input range, see x_safe below).  Both bounds scale with the row, so a
+  // network whose BatchNorms are rescaled by 2^k uploads the same blob.
+  float *bw0 = blob, *bb0 = blob + n_w0, *bw1 = blob + n_w0 + n_b0;
+  for (int u = 0; u < 3 * H; u++) {
+    double est = std::max(0.0, (double)bb0[u]), sw = 0, wmax = 0;
+    for (int k = 0; k < 5; k++) sw += fabs((double)bw0[u * 5 + k]);
+    est += PMI_X_NOM * sw;
+    for (int o = 0; o < H; o++) wmax = std::max(wmax, fabs((double)bw1[(size_t)u * H + o]));
+    if (!std::isfinite(est) || !std::isfinite(wmax)) continue;  // refused below
+    int s = 0, e2;
+    if (est > 0) {  // (an all-zero row keeps s = 0)
+      frexp(est, &e2);  // est = m * 2^e2, m in [0.5, 1): floor(log2(est)) = e2 - 1
+      s = PMI_BAL_T - (e2 - 1);
+    }
+#if TC_F16
+    if (wmax > 0) {  // smallest s with wmax * 2^-s * TC_WSCALE < 65504
+      frexp(wmax * TC_WSCALE / 65504.0, &e2);
+      s = std::max(s, e2);
+    }
+#endif
+    if (s == 0) continue;
+    // only an exact rescaling is applied (no value of the row or the column leaves fp32's normal range)
+    auto exact = [](float v, int e) { return ldexpf(ldexpf(v, e), -e) == v; };
+    bool ok = exact(bb0[u], s);
+    for (int k = 0; k < 5; k++) ok = ok && exact(bw0[u * 5 + k], s);
+    for (int o = 0; o < H; o++) ok = ok && exact(bw1[(size_t)u * H + o], -s);
+    if (!ok) continue;
+    for (int k = 0; k < 5; k++) bw0[u * 5 + k] = ldexpf(bw0[u * 5 + k], s);
+    bb0[u] = ldexpf(bb0[u], s);
+    for (int o = 0; o < H; o++) bw1[(size_t)u * H + o] = ldexpf(bw1[(size_t)u * H + o], -s);
+  }
+  // Range of the tensor path (fp16 operands): x_safe is the largest max_k |x_k| of a pair row for which every layer-0
+  // activation stays below fp16's largest finite value, with a 2^-8 margin for the fp32 rounding of the pre-activation;
+  // the kernel counts rows beyond it.  The tensor path serves the weights when every value is finite, every fc1 half is
+  // finite after the TC_WSCALE pre-scale and x_safe covers at least the nominal input bound PMI_X_NOM (in-map
+  // observations give pair inputs up to 16); otherwise the CUDA-core kernel does.
+  bool finite = std::isfinite(w->b2);
+  for (size_t k = 0; k < total; k++) finite = finite && std::isfinite(blob[k]);
+  float w1max = 0.f;
+  for (size_t k = 0; k < n_w1; k++) w1max = fmaxf(w1max, fabsf(bw1[k]));
+  double x_safe = DBL_MAX;
+#if TC_F16
+  for (int u = 0; u < 3 * H; u++) {
+    double sw = 0;
+    for (int k = 0; k < 5; k++) sw += fabs((double)bw0[u * 5 + k]);
+    if (sw > 0) x_safe = std::min(x_safe, std::max(0.0, 65504.0 * (1.0 - 1.0 / 256) - std::max(0.0, (double)bb0[u])) / sw);
+  }
+  const bool tc_range = finite && (double)w1max * TC_WSCALE < 65504.0 && x_safe >= PMI_X_NOM;
+#else
+  const bool tc_range = finite;
+#endif
   if (h->d_pmi_blob && h->pmi.H != H) { CUDA_TRY(cudaStreamSynchronize(st)); cudaFree(h->d_pmi_blob); h->d_pmi_blob = nullptr; }
   if (!h->d_pmi_blob) CUDA_TRY(cudaMalloc(&h->d_pmi_blob, total * sizeof(float)));
   CUDA_TRY(cudaMemcpyAsync(h->d_pmi_blob, blob, total * sizeof(float), cudaMemcpyHostToDevice, st));
   CUDA_TRY(cudaStreamSynchronize(st));
-  free(blob);
   h->pmi.H = H;
   h->pmi.w0 = h->d_pmi_blob;
   h->pmi.b0 = h->pmi.w0 + n_w0;
@@ -589,17 +659,28 @@ extern "C" int uavsim_set_pmi_weights(uavsim_t *h, const UavSimPmiWeights *w, vo
   const bool tc_shape = (H == 128 || H == 64);
   if (rc && !tc_shape) return rc;  // only the tensor path (hidden 64 / 128) can take over a shape the CUDA-core kernel cannot hold
   h->has_tc = false;
+  h->tc_range = tc_range;
+  h->has_pmi = true;
+  if (tc_shape && !tc_range) {
+    if (h->has_cc) return 0;  // the CUDA-core kernel serves these weights (automatic choice; path 2 is refused)
+    h->has_pmi = false;
+    SET_ERR("uavsim_set_pmi_weights: n_uav=%d needs the tensor-core PMI path, and these weights exceed its fp16 range "
+            "(after rebalancing: max |w1'| * %g = %g, pair-row input range %g < %g)", h->kp.n, (double)TC_WSCALE,
+            (double)w1max * TC_WSCALE, x_safe, PMI_X_NOM);
+    return UAVSIM_ERR_UNSUPPORTED;
+  }
   if (tc_shape) {
-    // tensor-core path: fc1 split hi/lo and laid out as the K-major UMMA tiles the kernel bulk-copies, chunk c, part
-    // {hi, lo}: fp16 (TC_F16, weights pre-scaled by TC_WSCALE): element (unit o, input k) at half (k/8)*(H*8) + o*8 + (k%8);
-    // TF32 (H = 128 only): at float (k/4)*512 + o*4 + (k%4)
+    // tensor-core path: fc1 (rebalanced, transposed in the blob) split hi/lo and laid out as the K-major UMMA tiles the
+    // kernel bulk-copies, chunk c, part {hi, lo}: fp16 (TC_F16, weights pre-scaled by TC_WSCALE): element (unit o, input
+    // k) at half (k/8)*(H*8) + o*8 + (k%8); TF32 (H = 128 only): at float (k/4)*512 + o*4 + (k%4)
     const int H3 = 3 * H, nchunk = H3 / TC_KC;
     const size_t tile = (size_t)H * TC_KC * (TC_F16 ? 2 : 4) / 4, total_t = (size_t)nchunk * 2 * tile;
-    float *tiles = (float *)malloc(total_t * sizeof(float));
+    std::vector<float> tiles_v(total_t);
+    float *tiles = tiles_v.data();
     for (int c = 0; c < nchunk; c++)
       for (int o = 0; o < H; o++)
         for (int kk = 0; kk < TC_KC; kk++) {
-          const float v = w->w1[(size_t)o * H3 + c * TC_KC + kk] * TC_WSCALE;
+          const float v = bw1[(size_t)(c * TC_KC + kk) * H + o] * TC_WSCALE;
 #if TC_F16
           const __half hi = __float2half_rn(v), lo = __float2half_rn(v - __half2float(hi));
           const size_t e = (size_t)(kk / 8) * ((size_t)H * 8) + (size_t)o * 8 + (kk % 8);
@@ -616,7 +697,6 @@ extern "C" int uavsim_set_pmi_weights(uavsim_t *h, const UavSimPmiWeights *w, vo
     CUDA_TRY(cudaMalloc(&h->d_tc_tiles, total_t * sizeof(float)));
     CUDA_TRY(cudaMemcpyAsync(h->d_tc_tiles, tiles, total_t * sizeof(float), cudaMemcpyHostToDevice, st));
     CUDA_TRY(cudaStreamSynchronize(st));
-    free(tiles);
     rc = raise_dynamic_smem(H == 64 ? (const void *)uavsim_pmi_tc_kernel<64> : (const void *)uavsim_pmi_tc_kernel<128>, h->device, TcSmem::total);
     if (rc) return rc;
     const int n = h->kp.n, per_env = n * (n - 1) > 0 ? n * (n - 1) : 1;
@@ -624,9 +704,9 @@ extern "C" int uavsim_set_pmi_weights(uavsim_t *h, const UavSimPmiWeights *w, vo
     if (G > TC_PMAX / per_env) G = TC_PMAX / per_env;
     if ((int64_t)G > h->E) G = (int)h->E;
     h->tc_g = G < 1 ? 1 : G;
+    h->tc_x_safe = (float)std::min(x_safe, (double)FLT_MAX);
     h->has_tc = true;
   }
-  h->has_pmi = true;
   return 0;
 }
 

@@ -11,7 +11,7 @@ import torch
 import torch.distributed as dist
 
 _SUM_KEYS = ("rewards", "target_tracking_reward", "boundary_punishment", "duplicate_tracking_punishment",
-             "covered_sum", "env_steps")
+             "covered_sum", "env_steps", "pmi_rows_out_of_range")
 
 
 def shard_envs(total_envs, rank, world_size):
@@ -27,11 +27,12 @@ def reduce_episode_stats(stats, device=None, group=None):
     if not (dist.is_available() and dist.is_initialized()) or dist.get_world_size(group) == 1:
         return dict(stats)
     dev = device if device is not None else ("cuda" if dist.get_backend(group) == "nccl" else "cpu")
-    s = torch.tensor([stats[k] for k in _SUM_KEYS], dtype=torch.float64, device=dev)
+    keys = [k for k in _SUM_KEYS if k in stats]  # (every rank passes the same keys)
+    s = torch.tensor([stats[k] for k in keys], dtype=torch.float64, device=dev)
     mx = torch.tensor([stats["covered_max"]], dtype=torch.float64, device=dev)
     dist.all_reduce(s, op=dist.ReduceOp.SUM, group=group)
     dist.all_reduce(mx, op=dist.ReduceOp.MAX, group=group)
-    out = {k: float(v) for k, v in zip(_SUM_KEYS, s.tolist())}
+    out = {k: float(v) for k, v in zip(keys, s.tolist())}
     out["covered_max"] = float(mx.item())
     return out
 

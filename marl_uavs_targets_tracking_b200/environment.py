@@ -413,13 +413,15 @@ class BatchedEnvironment:
 
     def episode_stats(self):
         """Sums accumulated on the device since the last reset (what src/train.py:181-192 accumulates):
-        dict with the four reward sums, covered sum / max and the number of env-steps."""
+        dict with the four reward sums, covered sum / max, the number of env-steps and `pmi_rows_out_of_range`: pair rows
+        the tensor-core PMI kernel saw with inputs beyond the range its fp16 activations hold (0 when it is exact)."""
         out = (C.c_double * 8)()
         with self._on_device():
             _cabi.check(self._lib.uavsim_episode_stats(self._h, out, self._stream()), "uavsim_episode_stats")
         v = list(out)
         return {"rewards": v[0], "target_tracking_reward": v[1], "boundary_punishment": v[2],
-                "duplicate_tracking_punishment": v[3], "covered_sum": v[4], "covered_max": v[5], "env_steps": v[6]}
+                "duplicate_tracking_punishment": v[3], "covered_sum": v[4], "covered_max": v[5], "env_steps": v[6],
+                "pmi_rows_out_of_range": v[7]}
 
     def launch_count(self):
         return int(self._lib.uavsim_launch_count(self._h)) if self._h is not None else 0
