@@ -174,9 +174,10 @@ int uavsim_set_pmi_path(uavsim_t *h, int path);
  * out[4] = sum of covered_targets over env-steps, out[5] = max covered_targets,
  * out[6] = env-steps accumulated, out[7] = pair rows the tensor-core PMI kernel evaluated with inputs beyond the range its
  * fp16 activations hold for the uploaded weights (their logits saturate; 0 in any run the tensor path serves exactly,
- * DESIGN.md section 3.2; the CUDA-core kernel has no such limit and never counts).  Synchronises `stream`.  The reward sums of the step kernels are
- * accumulated as integer counts of 2^-22 per (environment, UAV, step) -- exact in any order, so the totals are
- * bit-reproducible although CTAs draw their environments from a counter; resolution 2.4e-7 per value. */
+ * DESIGN.md section 3.2; the CUDA-core kernel has no such limit and never counts).  Synchronises `stream`.  Every kernel
+ * accumulates the reward sums as integer counts of 2^-22 of the float32 values it writes to rew4, one per (environment,
+ * UAV, step) -- exact in any order, so the totals are bit-reproducible although CTAs draw their environments from a
+ * counter, and do not depend on which kernel served a step; resolution 2.4e-7 per value. */
 int uavsim_episode_stats(uavsim_t *h, double out[8], void *stream);
 
 /* number of kernels this handle has launched (bench.py reports it as gpu_launches) */

@@ -65,51 +65,26 @@ __global__ void uavsim_random_actions_kernel(const KParams P, int32_t *__restric
   }
 }
 
-__global__ void uavsim_stats_clear_kernel(double *stats, int count) {
-  for (int k = blockIdx.x * blockDim.x + threadIdx.x; k < count; k += gridDim.x * blockDim.x) stats[k] = 0.0;
+__global__ void uavsim_stats_clear_kernel(long long *stats, int count) {
+  for (int k = blockIdx.x * blockDim.x + threadIdx.x; k < count; k += gridDim.x * blockDim.x) stats[k] = 0;
 }
 
-// fixed-order reduction of the per-CTA slots: one CTA of 256 threads, strided partial sums then a shared-memory
-// tree (the association order depends only on `slots`, so totals are reproducible)
-__global__ void uavsim_stats_reduce_kernel(const double *__restrict__ partial, int slots, double *__restrict__ out) {
-  __shared__ double sh[256][STAT_W];
-  if (blockIdx.x != 0) return;
-  double a[STAT_W] = {0, 0, 0, 0, 0, 0, 0, 0};
-  for (int s = threadIdx.x; s < 2 * slots; s += 256) {
-    const double *p = partial + (size_t)s * STAT_W;
-    for (int k = 0; k < 5; k++) a[k] += p[k];
-    a[5] = fmax(a[5], p[5]);
-    a[6] += p[6];
-  }
-  {  // third region: the fast step kernel's reward sums as 64-bit counts of 2^-22 (exact in any order)
-    const long long *fx = reinterpret_cast<const long long *>(partial + (size_t)2 * slots * STAT_W);
-    // (field 4: pair rows the tensor PMI kernel found beyond its fp16 range, a plain count -> out[7])
-    long long c[5] = {0, 0, 0, 0, 0};
-    for (int s = threadIdx.x; s < slots; s += 256)
-      for (int k = 0; k < 5; k++) c[k] += fx[(size_t)s * STAT_W + k];
-    __shared__ long long shc[256][5];
-    for (int k = 0; k < 5; k++) shc[threadIdx.x][k] = c[k];
-    __syncthreads();
-    for (int w = 128; w > 0; w >>= 1) {
-      if ((int)threadIdx.x < w)
-        for (int k = 0; k < 5; k++) shc[threadIdx.x][k] += shc[threadIdx.x + w][k];
-      __syncthreads();
-    }
-    if (threadIdx.x == 0) {
-      for (int k = 0; k < 4; k++) a[k] += (double)shc[0][k] * (1.0 / 4194304.0);
-      a[7] = (double)shc[0][4];
-    }
-  }
-  for (int k = 0; k < STAT_W; k++) sh[threadIdx.x][k] = a[k];
+// Combines the per-CTA slots (common.cuh: ST_*) in one CTA: integer sums and a maximum, exact in any order; the four
+// reward counts scale by 2^-22.
+__global__ void uavsim_stats_reduce_kernel(const long long *__restrict__ stats, int slots, double *__restrict__ out) {
+  __shared__ long long tot[STAT_W];
+  if (threadIdx.x < STAT_W) tot[threadIdx.x] = 0;
   __syncthreads();
-  for (int w = 128; w > 0; w >>= 1) {
-    if ((int)threadIdx.x < w) {
-      for (int k = 0; k < 5; k++) sh[threadIdx.x][k] += sh[threadIdx.x + w][k];
-      sh[threadIdx.x][5] = fmax(sh[threadIdx.x][5], sh[threadIdx.x + w][5]);
-      sh[threadIdx.x][6] += sh[threadIdx.x + w][6];
-      sh[threadIdx.x][7] += sh[threadIdx.x + w][7];
+  long long a[STAT_W] = {0, 0, 0, 0, 0, 0, 0, 0};
+  for (int s = threadIdx.x; s < slots; s += blockDim.x)
+    for (int k = 0; k < STAT_W; k++) {
+      const long long v = stats[(size_t)s * STAT_W + k];
+      a[k] = (k == ST_CMAX) ? max(a[k], v) : a[k] + v;
     }
-    __syncthreads();
+  for (int k = 0; k < STAT_W; k++) {
+    if (k == ST_CMAX) atomicMax(&tot[k], a[k]);
+    else atomicAdd(reinterpret_cast<unsigned long long *>(&tot[k]), (unsigned long long)a[k]);
   }
-  if (threadIdx.x < STAT_W) out[threadIdx.x] = sh[0][threadIdx.x];
+  __syncthreads();
+  if (threadIdx.x < STAT_W) out[threadIdx.x] = (double)tot[threadIdx.x] * (threadIdx.x <= ST_DUP ? 1.0 / 4194304.0 : 1.0);
 }

@@ -11,7 +11,10 @@
 #include "philox.cuh"
 
 #define PMI_NT 256   // threads per CTA, PMI kernel
-#define STAT_W 8     // doubles per statistics slot
+
+// Fields of a statistics slot (int64): 0-3 the four reward planes as sf_fx counts of the fp32 values written to rew4,
+// then covered targets (sum), their maximum, env-steps and the PMI pair rows beyond the tensor path's fp16 range.
+enum { ST_REW, ST_TT, ST_BP, ST_DUP, ST_COV, ST_CMAX, ST_ENVS, ST_PMI_OOR, STAT_W };
 
 static thread_local char g_err[512] = "";
 #define SET_ERR(...) snprintf(g_err, sizeof(g_err), __VA_ARGS__)
@@ -67,9 +70,8 @@ struct KParams {
   float k_ex1_f, tv_over_uv_f, cx_f, cy_f;
   float dtv_u_f;  // dt*v_max of the UAVs in fp32
   const double *sincos_tab;  // [FM_TAB_SIZE][2] sine / cosine of k pi/32 (fast_math.cuh), device memory
-  int stat_slots;            // slots per region of the statistics array
   int *fast_ctr;             // counter-scheduled kernels (fast / generic step, PMI tensor): {next unit of work beyond the first
-                             // wave, CTAs that have left}; zero between launches (the last CTA to leave rewinds it); launches of one
+                             // wave, CTAs that have left}; zero between launches (work_counter_leave rewinds it); launches of one
                              // handle are stream-ordered, so one pair serves all of them
 };
 
@@ -80,13 +82,13 @@ struct PmiDev {
 };
 
 typedef void (*StepKernelFn)(const KParams, const UavSimBuffers, const double *, int64_t, int64_t, int, int, double,
-                             int, double *);
+                             int, long long *);
 struct ActEntry;
 typedef void (*FastKernelFn)(const KParams, const UavSimBuffers, const ActEntry *, int64_t, int64_t, int, double, int,
-                             double *);
+                             long long *);
 
 typedef void (*SmallKernelFn)(const KParams, const UavSimBuffers, const ActEntry *, int64_t, int64_t, int, double, int,
-                              double *, int, uint64_t, uint32_t);
+                              long long *, int, uint64_t, uint32_t);
 
 struct PmiTcDev;
 
@@ -98,7 +100,7 @@ struct uavsim {
   int device, sm_count;
   int64_t E;
   double *d_dth;      // [3*na] dt * heading-rate per action (src/agent/uav.py:73-81,96), its cos and sin
-  double *d_stats;    // [3][slots][STAT_W] per-CTA partial sums (step kernel | pmi kernel | fast step kernel: int64 counts of 2^-22)
+  long long *d_stats; // [stat_slots][STAT_W] per-CTA statistics, slot = block index (every step and PMI kernel)
   double *d_stats8;   // [8] reduced
   double *h_stats8;   // pinned
   int stat_slots;
@@ -167,67 +169,39 @@ __device__ __forceinline__ double clipnorm_m1(double v, double lo) {
   return (v - lo) / (0.0 - lo) - 1.0;
 }
 
-__device__ __forceinline__ double warp_sum(double v) {
-#pragma unroll
-  for (int o = 16; o > 0; o >>= 1) v += __shfl_down_sync(0xffffffffu, v, o);
-  return v;
-}
-__device__ __forceinline__ int warp_max(int v) {
-#pragma unroll
-  for (int o = 16; o > 0; o >>= 1) v = max(v, __shfl_down_sync(0xffffffffu, v, o));
-  return v;
-}
-
-// Block-wide reduction of per-thread statistics into this CTA's slot (accumulating across launches;
-// one writer per slot, no atomics, so the totals are reproducible for a fixed launch geometry).
-// Statistics of kernels whose CTAs draw their work from a launch-wide counter (KParams::fast_ctr): which CTA steps
-// which environment depends on timing, so the reward sums are kept as integer counts of 2^-22 -- exact, hence the same
-// totals whatever the grouping.  A value in [-1, 1] as such a count: v + 3 lies in [2, 4], where consecutive floats are
-// 2^-22 apart and the bit pattern is linear in the value (round to nearest even): FADD + IADD3.
+// Episode statistics.  Which CTA steps which environment depends on timing wherever the work comes from a launch-wide
+// counter (KParams::fast_ctr), so every kernel keeps its statistics as integers: the reward values as counts of 2^-22,
+// covered targets and env-steps as plain counts.  Integer sums are exact in any order, hence the totals are the same
+// whatever the grouping and whichever kernel served a step.  A value in [-1, 1] as such a count: v + 3 lies in [2, 4],
+// where consecutive floats are 2^-22 apart and the bit pattern is linear in the value (round to nearest even): FADD + IADD3.
 __device__ __forceinline__ int sf_fx(float v) { return __float_as_int(v + 3.0f) - 0x40400000; }
 
-// the four reward sums as 64-bit fixed-point counts
-__device__ inline void block_stats_commit_fx(long long *red /*smem [warps][4]*/, long long *slot, long long v0, long long v1, long long v2,
-                                             long long v3) {
-  const int lane = threadIdx.x & 31, wid = threadIdx.x >> 5;
-  for (int o = 16; o > 0; o >>= 1) {
-    v0 += __shfl_xor_sync(0xffffffffu, v0, o); v1 += __shfl_xor_sync(0xffffffffu, v1, o);
-    v2 += __shfl_xor_sync(0xffffffffu, v2, o); v3 += __shfl_xor_sync(0xffffffffu, v3, o);
-  }
-  __syncthreads();
-  const int nw = (int)(blockDim.x >> 5);   // (red holds [nw][4]: the callers' 64-entry buffers serve up to 16 warps)
-  if (lane == 0) { red[wid * 4 + 0] = v0; red[wid * 4 + 1] = v1; red[wid * 4 + 2] = v2; red[wid * 4 + 3] = v3; }
-  __syncthreads();
-  if (threadIdx.x < 4) {
-    long long a = 0;
-    for (int w = 0; w < nw; w++) a += red[w * 4 + threadIdx.x];
-    slot[threadIdx.x] += a;
-  }
-  __syncthreads();
-}
-
-__device__ void block_stats_commit(double *red /*smem [nwarps*7], at most 64 doubles: 9 warps*/, double *slot, double v0, double v1, double v2,
-                                   double v3, double v4, int vmax, double v6, int nthreads) {
-  const int lane = threadIdx.x & 31, wid = threadIdx.x >> 5, nw = nthreads >> 5;
-  v0 = warp_sum(v0); v1 = warp_sum(v1); v2 = warp_sum(v2); v3 = warp_sum(v3); v4 = warp_sum(v4);
-  v6 = warp_sum(v6);
-  vmax = warp_max(vmax);
-  __syncthreads();
-  if (lane == 0) {
-    red[wid * 7 + 0] = v0; red[wid * 7 + 1] = v1; red[wid * 7 + 2] = v2; red[wid * 7 + 3] = v3;
-    red[wid * 7 + 4] = v4; red[wid * 7 + 5] = (double)vmax; red[wid * 7 + 6] = v6;
-  }
-  __syncthreads();
-  if (threadIdx.x == 0) {
-    double a[7] = {0, 0, 0, 0, 0, 0, 0};
-    for (int w = 0; w < nw; w++) {
-      for (int k = 0; k < 5; k++) a[k] += red[w * 7 + k];
-      a[5] = fmax(a[5], red[w * 7 + 5]);
-      a[6] += red[w * 7 + 6];
+// Adds the statistics of the calling warp's lanes to `slot` (the CTA's slot of the statistics array, accumulating across
+// launches).  Every lane of the warp calls; lanes and fields without a value pass 0.  Lane 0 adds the warp's totals with
+// 64-bit atomics (the maximum for ST_CMAX), skipping zeros: no shared memory, no barrier.
+__device__ __forceinline__ void stats_commit(long long *slot, long long rew, long long tt, long long bp, long long dup,
+                                             long long cov, long long cmax, long long envs, long long pmi_oor = 0) {
+  long long v[STAT_W] = {rew, tt, bp, dup, cov, cmax, envs, pmi_oor};
+#pragma unroll
+  for (int k = 0; k < STAT_W; k++)
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) {
+      const long long w = __shfl_xor_sync(0xffffffffu, v[k], o);
+      v[k] = (k == ST_CMAX) ? max(v[k], w) : v[k] + w;
     }
-    for (int k = 0; k < 5; k++) slot[k] += a[k];
-    slot[5] = fmax(slot[5], a[5]);
-    slot[6] += a[6];
+  if ((threadIdx.x & 31) != 0) return;
+#pragma unroll
+  for (int k = 0; k < STAT_W; k++) {
+    if (v[k] == 0) continue;
+    if (k == ST_CMAX) atomicMax(slot + k, v[k]);
+    else atomicAdd(reinterpret_cast<unsigned long long *>(slot + k), (unsigned long long)v[k]);
   }
 }
 
+// End of a counter-scheduled launch (KParams::fast_ctr): thread 0 of every CTA signs out after its last unit of work,
+// and the last CTA to leave rewinds the counter for the next launch.
+__device__ __forceinline__ void work_counter_leave(int *ctr) {
+  if (threadIdx.x != 0) return;
+  __threadfence();
+  if (atomicAdd(ctr + 1, 1) == (int)gridDim.x - 1) { ctr[0] = 0; ctr[1] = 0; __threadfence(); }
+}

@@ -13,7 +13,6 @@
 struct PmiSmem {
   float *obs;       // [G*n*12]
   double *raw;      // [G*n]
-  double *red;      // [64]
   uint32_t *off;    // [G*n+1]
   uint32_t *pair;   // [pmax]  (a << 16) | b, local UAV indices in the group
   float *logit;     // [pmax]
@@ -25,7 +24,7 @@ struct PmiSmem {
 
 static size_t pmi_smem_bytes(int n, int H, int G, int pmax, int TM) {
   size_t b = 0;
-  b += (size_t)G * n * 8 + 64 * 8;                 // raw, red (doubles first)
+  b += (size_t)G * n * 8;                          // raw (doubles first)
   b += (size_t)G * n * 12 * 4;                     // obs
   b += ((size_t)G * n + 1 + 3) / 4 * 4 * 4;        // off (padded)
   b += (size_t)pmax * 8;                           // pair + logit
@@ -38,7 +37,6 @@ __device__ __forceinline__ PmiSmem pmi_carve(unsigned char *base, int n, int H, 
   PmiSmem s;
   double *d = reinterpret_cast<double *>(base);
   s.raw = d; d += (size_t)G * n;
-  s.red = d; d += 64;
   float *f = reinterpret_cast<float *>(d);
   s.obs = f; f += (size_t)G * n * 12;
   s.off = reinterpret_cast<uint32_t *>(f); f += ((size_t)G * n + 1 + 3) / 4 * 4;
@@ -57,7 +55,7 @@ __device__ __forceinline__ PmiSmem pmi_carve(unsigned char *base, int n, int H, 
 template <int CPT, int TM>  // H = 16*CPT output columns; TM rows per tile (TM/16 rows per thread)
 __global__ void __launch_bounds__(PMI_NT)
 uavsim_pmi_kernel(const KParams P, const UavSimBuffers B, const PmiDev W, int64_t env_begin, int64_t env_count,
-                  int G, int pmax, double coop, double *__restrict__ stats_partial) {
+                  int G, int pmax, double coop, long long *__restrict__ stats) {
   constexpr int H = 16 * CPT, H3 = 3 * H, LD0 = H3 + 4, RPT = TM / 16;
   extern __shared__ __align__(16) unsigned char smem_raw[];
   const int n = P.n, tid = threadIdx.x;
@@ -69,7 +67,7 @@ uavsim_pmi_kernel(const KParams P, const UavSimBuffers B, const PmiDev W, int64_
 
   const int ty = tid >> 4, tx = tid & 15;
   const int64_t ngroups = (env_count + G - 1) / G;
-  double st_r = 0;
+  long long fx_r = 0;  // reward statistic (common.cuh: sf_fx)
 
   for (int64_t grp = blockIdx.x; grp < ngroups; grp += gridDim.x) {
     const int64_t e0 = env_begin + grp * G;
@@ -188,9 +186,9 @@ uavsim_pmi_kernel(const KParams P, const UavSimBuffers B, const PmiDev W, int64_
       }
       r = fmin(fmax(r, -1.0), 1.0);
       B.rew4[e0 * n + tid] = (float)r;
-      st_r += r;
+      fx_r += sf_fx((float)r);
     }
   }
-  block_stats_commit(S.red, stats_partial + (size_t)blockIdx.x * STAT_W, st_r, 0, 0, 0, 0, 0, 0, PMI_NT);
+  stats_commit(stats + (size_t)blockIdx.x * STAT_W, fx_r, 0, 0, 0, 0, 0, 0);
 }
 

@@ -107,8 +107,7 @@ struct TcSmem {  // byte offsets inside dynamic shared memory (base is 1024-byte
   static constexpr uint32_t part = w0 + (TC_H3 / 2) * 12 * 4;          // float [TC_PARTS-1][2][128] fc2 partial dots of the other threads of a row
   static constexpr uint32_t b1 = part + (TC_PARTS - 1) * TC_SET * 128 * 4;   // float [128]
   static constexpr uint32_t w2 = b1 + TC_H * 4;                          // float [128]
-  static constexpr uint32_t red = w2 + TC_H * 4;                         // double [7 per warp]
-  static constexpr uint32_t bar = red + (TC_NT / 32) * 7 * 8;            // 3 x TC_NS + 2 mbarriers + tmem pointer
+  static constexpr uint32_t bar = w2 + TC_H * 4;                         // 3 x TC_NS + 2 mbarriers + tmem pointer
   static constexpr uint32_t total = bar + 128;
 };
 static_assert(TcSmem::total <= 232448, "tensor PMI kernel: shared memory over the 227 KB per-CTA limit");
@@ -245,7 +244,7 @@ struct PmiTcDev {
 template <int H>   // hidden size of the PMI network: 128 (src/configs/*.yaml) or 64 (the default of PMINetwork's constructor)
 __global__ void __launch_bounds__(TC_NT, 1)
 uavsim_pmi_tc_kernel(const KParams P, const UavSimBuffers B, const PmiTcDev W, int64_t env_begin, int64_t env_count,
-                     int G, double coop, double *__restrict__ stats_partial) {
+                     int G, double coop, long long *__restrict__ stats) {
   static_assert(H == 64 || H == 128, "tensor PMI kernel: hidden size 64 or 128");
   constexpr int H3 = 3 * H, NCHUNK = H3 / TC_KC;
   constexpr uint32_t A_BYTES = (uint32_t)H * TC_KC * (TC_F16 ? 2 : 4);   // one H x TC_KC weight block (hi or lo)
@@ -265,7 +264,6 @@ uavsim_pmi_tc_kernel(const KParams P, const UavSimBuffers B, const PmiTcDev W, i
   float *s_part = reinterpret_cast<float *>(smem + TcSmem::part);
   float *s_b1 = reinterpret_cast<float *>(smem + TcSmem::b1);
   float *s_w2 = reinterpret_cast<float *>(smem + TcSmem::w2);
-  double *s_red = reinterpret_cast<double *>(smem + TcSmem::red);
   uint32_t *s_tmem = reinterpret_cast<uint32_t *>(smem + TcSmem::bar + 120);
   const uint32_t sbase = smem_u32(smem);
   const uint32_t bar0 = sbase + TcSmem::bar;
@@ -603,16 +601,6 @@ uavsim_pmi_tc_kernel(const KParams P, const UavSimBuffers B, const PmiTcDev W, i
   }
   __syncthreads();
   if (warp == 0) asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem_d), "r"(512u) : "memory");
-  if (tid == 0) {
-    __threadfence();
-    if (atomicAdd(P.fast_ctr + 1, 1) == (int)gridDim.x - 1) { P.fast_ctr[0] = 0; P.fast_ctr[1] = 0; __threadfence(); }
-  }
-  // (stats_partial is the PMI region of the statistics array; the fixed-point region follows it)
-  long long *const slot = reinterpret_cast<long long *>(stats_partial + (size_t)P.stat_slots * STAT_W) + (size_t)blockIdx.x * STAT_W;
-  block_stats_commit_fx(reinterpret_cast<long long *>(s_red), slot, fx_r, 0, 0, 0);
-  // field 4: pair rows out of the fp16 range (integer, so the order of the warps' additions does not matter)
-  if (producer) {
-    const int c = __reduce_add_sync(0xffffffffu, oor);
-    if (lane == 0 && c) atomicAdd(reinterpret_cast<unsigned long long *>(slot + 4), (unsigned long long)c);
-  }
+  work_counter_leave(P.fast_ctr);
+  stats_commit(stats + (size_t)blockIdx.x * STAT_W, fx_r, 0, 0, 0, 0, 0, 0, oor);
 }

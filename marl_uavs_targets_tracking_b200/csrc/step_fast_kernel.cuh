@@ -427,8 +427,7 @@ __device__ __noinline__ void sf_dup_checked(const FastSmem<N, M, AUX> *Sp, const
 template <int N, int M, bool AUX>
 __global__ void __launch_bounds__(FAST_NT, FAST_CTAS_PER_SM)
 uavsim_step_fast_kernel(const KParams P, const UavSimBuffers B, const ActEntry *__restrict__ act_tab, int64_t env_begin,
-                        int64_t env_count, int mode, double coop, int done_flag, double *__restrict__ stats_partial) {
-  long long *const stats_fx = reinterpret_cast<long long *>(stats_partial + 2 * (size_t)P.stat_slots * STAT_W);  // third region
+                        int64_t env_count, int mode, double coop, int done_flag, long long *__restrict__ stats) {
   static_assert(N == 64 && M == 64 && FAST_NT == 64, "one thread per UAV and per target");
   typedef FastSmem<N, M, AUX> SmemT;
   static_assert(offsetof(SmemT, sloto) - offsetof(SmemT, slotn) == sizeof(SlotRec) * (N / 2), "record offset");
@@ -468,12 +467,10 @@ uavsim_step_fast_kernel(const KParams P, const UavSimBuffers B, const ActEntry *
   const int64_t plane = P.E * N;
   const float inv_dp_f = P.inv_dp_f, inv_dc_f = P.inv_dc_f, inv_na_f = P.inv_na_f;
   const float k_ex0 = 1.4426950408889634f, k_ex1 = P.k_ex1_f;
-  // Statistics of the four reward planes as FIXED-POINT sums (2^-22 per count, FastFx): which CTA takes which
-  // environment depends on timing, and only integer sums give the same totals whatever the grouping.  Coverage and
-  // environment counts are integers in fp64 (exact in any order).
+  // statistics (common.cuh: sf_fx); the reward counts are summed in 32 bits for up to 256 environments
   int fx_r = 0, fx_tt = 0, fx_bp = 0, fx_dup = 0;                 // at most 2^22 per environment
   long long fxs_r = 0, fxs_tt = 0, fxs_bp = 0, fxs_dup = 0;
-  double st_cov = 0, st_envs = 0;
+  long long st_cov = 0, st_envs = 0;
   int st_cmax = 0;
   uint32_t trips = 0;
   uint32_t parity = 0;
@@ -812,7 +809,7 @@ uavsim_step_fast_kernel(const KParams P, const UavSimBuffers B, const ActEntry *
       if (lane == 0) { S.cover[warp][0] = c0; S.cover[warp][1] = c1; }
     }
 
-    // The terms below only feed fp32 outputs (and fp64 statistics of those outputs): evaluated in fp32.  The one
+    // The terms below only feed fp32 outputs (and the statistics of those outputs): evaluated in fp32.  The one
     // decision among them, inside / outside the map (uav.py:239), stays in fp64.
     float raw, ttn, bpn, dupn;
     {
@@ -904,22 +901,16 @@ uavsim_step_fast_kernel(const KParams P, const UavSimBuffers B, const ActEntry *
       const int c = __popc(S.cover[0][0] | S.cover[1][0]) + __popc(S.cover[0][1] | S.cover[1][1]);
       B.covered[e] = c;
       if (B.done) B.done[e] = done_flag;
-      st_cov += (double)c;
+      st_cov += c;
       st_cmax = max(st_cmax, c);
-      st_envs += 1.0;
+      st_envs++;
     }
   }
   __syncwarp();
   if (warp == 0) {
     if (elect_one()) asm volatile("cp.async.bulk.wait_group 0;" ::: "memory");  // outputs complete before the CTA retires
   }
-  if (t == 0) {  // the last CTA to leave rewinds the counter for the next launch
-    __threadfence();
-    if (atomicAdd(P.fast_ctr + 1, 1) == (int)gridDim.x - 1) { P.fast_ctr[0] = 0; P.fast_ctr[1] = 0; __threadfence(); }
-  }
-  __syncthreads();
-  fxs_r += fx_r; fxs_tt += fx_tt; fxs_bp += fx_bp; fxs_dup += fx_dup;
-  block_stats_commit_fx(reinterpret_cast<long long *>(S.ux), stats_fx + (size_t)blockIdx.x * STAT_W, fxs_r, fxs_tt, fxs_bp, fxs_dup);
-  block_stats_commit(reinterpret_cast<double *>(S.ux), stats_partial + (size_t)blockIdx.x * STAT_W, 0.0, 0.0, 0.0, 0.0, st_cov,
-                     st_cmax, st_envs, FAST_NT);
+  work_counter_leave(P.fast_ctr);
+  stats_commit(stats + (size_t)blockIdx.x * STAT_W, fxs_r + fx_r, fxs_tt + fx_tt, fxs_bp + fx_bp, fxs_dup + fx_dup, st_cov,
+               st_cmax, st_envs);
 }

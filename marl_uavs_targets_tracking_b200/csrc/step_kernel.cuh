@@ -60,7 +60,7 @@ struct CtaSmem {
   unsigned char *env;  // [epb] environment blocks
   double *raw;         // [epb*n]
   double *dth;         // [3*na] per action: dt*rate, cos(dt*rate), sin(dt*rate)
-  double *red;         // [64]
+  long long *next;     // the group this CTA steps next (drawn by thread 0)
   float *obs;          // [epb*n*12]
   int *tcnt;           // [epb*m] UAVs strictly within dp of each target
   int *far;            // [epb] 1 if an entity is farther than KParams::rmax from the map centre
@@ -70,7 +70,7 @@ struct CtaSmem {
 static size_t step_smem_bytes(int n, int m, int na, int epb) {
   const EnvLayout L = env_layout(n, m);
   size_t b = (size_t)epb * L.stride;
-  b += ((size_t)epb * n + 64) * 8 + 8;          // raw, red (+ pad)
+  b += ((size_t)epb * n + 1) * 8 + 8;           // raw, next (+ pad)
   b += (size_t)epb * n * 12 * 4;                // obs
   b += ((size_t)epb * m + 2 * (size_t)epb) * 4 + 4;  // tcnt, far, cov (+ pad)
   b += 3 * (size_t)na * 8;                      // dth
@@ -84,8 +84,8 @@ __device__ __forceinline__ CtaSmem carve(unsigned char *base, int n, int m, int 
   s.env = base;
   double *d = reinterpret_cast<double *>(base + (size_t)epb * stride);  // stride is a multiple of 16
   s.raw = d; d += (size_t)epb * n;
-  s.red = d; d += 64;
-  d += ((size_t)epb * n) & 1;  // keep obs 16-byte aligned (plain pointer arithmetic: stays shared)
+  s.next = reinterpret_cast<long long *>(d); d += 1;
+  d += ((size_t)epb * n + 1) & 1;  // keep obs 16-byte aligned (plain pointer arithmetic: stays shared)
   s.obs = reinterpret_cast<float *>(d);
   int *ip = reinterpret_cast<int *>(s.obs + (size_t)epb * n * 12);
   s.tcnt = ip; ip += (size_t)epb * m;
@@ -479,9 +479,8 @@ template <int CN, int CM, bool MASKS, int NT>
 __global__ void __launch_bounds__(NT, UAVSIM_WARPS_PER_SM * 32 / NT)
 uavsim_step_kernel(const KParams P, const UavSimBuffers B, const double *__restrict__ g_dth, int64_t env_begin,
                    int64_t env_count, int epb_rt, int mode, double coop, int done_flag,
-                   double *__restrict__ stats_partial) {
+                   long long *__restrict__ stats) {
   extern __shared__ __align__(16) unsigned char smem_raw[];
-  static_assert((NT / 32) * 7 <= 64, "block_stats_commit: the 64-double reduction buffer holds 7 values per warp");
   const int n = CN ? CN : P.n, m = CM ? CM : P.m;
   const int epb = CN ? NT / CN : epb_rt;  // environments per CTA: the host passes NT / n, a constant when n is
   constexpr bool WARP_ENV = (CN > 0) && (CN % 32 == 0);
@@ -500,11 +499,9 @@ uavsim_step_kernel(const KParams P, const UavSimBuffers B, const double *__restr
 
   const int64_t ngroups = (env_count + epb - 1) / epb;
   // per-thread statistics, reduced once at the end (src/train.py:181-192)
-  // (reward sums as fixed-point counts: the groups beyond the first wave come from a launch-wide counter, common.cuh)
   long long fx_r = 0, fx_tt = 0, fx_bp = 0, fx_dup = 0;
-  double st_cov = 0, st_envs = 0;
+  long long st_cov = 0, st_envs = 0;
   int st_cmax = 0;
-  long long *const s_next = reinterpret_cast<long long *>(S.red + 63);  // (the reduction buffer is idle inside the loop)
 
   // Groups beyond the first wave are handed out by a launch-wide counter, as in the fast kernel: the warp schedulers
   // favour some CTAs, and with a fixed stride the favoured ones retire early and leave their SM under-occupied.
@@ -514,9 +511,9 @@ uavsim_step_kernel(const KParams P, const UavSimBuffers B, const double *__restr
     const int64_t e0 = env_begin + grp * epb;
     const int ne = (int)min((int64_t)epb, env_begin + env_count - e0);
     if (tid < epb) { S.far[tid] = 0; S.cov[tid] = 0; }  // (their readers of the previous iteration have passed a barrier)
-    if (tid == 0) *s_next = drawn;
+    if (tid == 0) *S.next = drawn;
     __syncthreads();                // previous iteration's readers are done; dth table visible
-    grp_next = *s_next;
+    grp_next = *S.next;
 #ifdef GENERIC_STATIC_STRIDE   // A/B switch: the fixed stride of round 1
     grp_next = grp + gridDim.x;
 #endif
@@ -679,16 +676,11 @@ uavsim_step_kernel(const KParams P, const UavSimBuffers B, const double *__restr
       const int c = S.cov[tid];
       B.covered[e0 + tid] = c;
       if (B.done) B.done[e0 + tid] = done_flag;
-      st_cov += (double)c;
+      st_cov += c;
       st_cmax = max(st_cmax, c);
-      st_envs += 1.0;
+      st_envs++;
     }
   }
-  if (tid == 0) {  // the last CTA to leave rewinds the counter for the next launch
-    __threadfence();
-    if (atomicAdd(P.fast_ctr + 1, 1) == (int)gridDim.x - 1) { P.fast_ctr[0] = 0; P.fast_ctr[1] = 0; __threadfence(); }
-  }
-  block_stats_commit_fx(reinterpret_cast<long long *>(S.red), reinterpret_cast<long long *>(stats_partial + 2 * (size_t)P.stat_slots * STAT_W) + (size_t)blockIdx.x * STAT_W,
-                        fx_r, fx_tt, fx_bp, fx_dup);
-  block_stats_commit(S.red, stats_partial + (size_t)blockIdx.x * STAT_W, 0.0, 0.0, 0.0, 0.0, st_cov, st_cmax, st_envs, NT);
+  work_counter_leave(P.fast_ctr);
+  stats_commit(stats + (size_t)blockIdx.x * STAT_W, fx_r, fx_tt, fx_bp, fx_dup, st_cov, st_cmax, st_envs);
 }

@@ -60,7 +60,7 @@ __host__ __device__ inline int small_group(int n, int m) {
 template <bool AUX>
 __global__ void __launch_bounds__(SMALL_NT, SMALL_CTAS_PER_SM)
 uavsim_step_small_kernel(const KParams P, const UavSimBuffers B, const ActEntry *__restrict__ act_tab, int64_t env_begin,
-                         int64_t env_count, int mode, double coop, int done_flag, double *__restrict__ stats_partial,
+                         int64_t env_count, int mode, double coop, int done_flag, long long *__restrict__ stats,
                          int rng_on, uint64_t rng_seed, uint32_t rng_step) {
   __shared__ SmallSmem S;
   const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
@@ -75,7 +75,7 @@ uavsim_step_small_kernel(const KParams P, const UavSimBuffers B, const ActEntry 
   const int gu = (int)(((float)lane + 0.5f) * __frcp_rn((float)n)), iu = lane - gu * n;
   const int gt = (int)(((float)lane + 0.5f) * __frcp_rn((float)m)), jt = lane - gt * m;
   const float k_ex0 = 1.4426950408889634f, k_ex1 = P.k_ex1_f;
-  double st_r = 0, st_tt = 0, st_bp = 0, st_dup = 0, st_cov = 0, st_envs = 0;
+  long long fx_r = 0, fx_tt = 0, fx_bp = 0, fx_dup = 0, st_cov = 0, st_envs = 0;  // statistics (common.cuh: sf_fx)
   int st_cmax = 0;
   // Programmatic dependent launch: when the steps of a rollout are queued back to back (uavsim_run_random_policy) this
   // grid may start while its predecessor drains -- everything above (parameters, lane roles) overlaps the predecessor's
@@ -296,11 +296,11 @@ uavsim_step_small_kernel(const KParams P, const UavSimBuffers B, const ActEntry 
           B.nbr_bits[gi * 2 + 1] = 0;
         }
         r = fmin(fmax(r, -1.0), 1.0);  // clip_and_normalize(reward, -1, 1) is a plain clip
-        if (!pmi_pending) { B.rew4[gi] = (float)r; st_r += r; }
+        if (!pmi_pending) { B.rew4[gi] = (float)r; fx_r += sf_fx((float)r); }
         B.rew4[plane + gi] = (float)ttn;
         B.rew4[2 * plane + gi] = (float)bpn;
         B.rew4[3 * plane + gi] = (float)dupn;
-        st_tt += ttn; st_bp += bpn; st_dup += dupn;
+        fx_tt += sf_fx((float)ttn); fx_bp += sf_fx((float)bpn); fx_dup += sf_fx((float)dupn);
         float4 *ob = reinterpret_cast<float4 *>(B.obs + gi * 12);
         ob[0] = make_float4(ob0, ob1, ob2, ob3);
         ob[1] = make_float4(ob4, H.tb0, H.tb1, H.tb2);
@@ -310,32 +310,14 @@ uavsim_step_small_kernel(const KParams P, const UavSimBuffers B, const ActEntry 
         const int c = __popc(S.cov[lane]);
         B.covered[e0 + lane] = c;
         if (B.done) B.done[e0 + lane] = done_flag;
-        st_cov += (double)c;
+        st_cov += c;
         st_cmax = max(st_cmax, c);
-        st_envs += 1.0;
+        st_envs++;
       }
     } else if (B.tracker_cnt && gt < ne) {
       B.tracker_cnt[(e0 + gt) * m + jt] = S.tcnt[gt][jt];
     }
   }
-  // episode statistics of the CTA: warp 0 holds them all (coverage on its first SMALL_G lanes); one writer per slot,
-  // fixed order
-  if (warp == 0) {
-#pragma unroll
-    for (int o = 16; o > 0; o >>= 1) {
-      st_r += __shfl_down_sync(0xffffffffu, st_r, o); st_tt += __shfl_down_sync(0xffffffffu, st_tt, o);
-      st_bp += __shfl_down_sync(0xffffffffu, st_bp, o); st_dup += __shfl_down_sync(0xffffffffu, st_dup, o);
-    }
-#pragma unroll
-    for (int o = SMALL_G / 2; o > 0; o >>= 1) {
-      st_cov += __shfl_down_sync(0xffffffffu, st_cov, o); st_envs += __shfl_down_sync(0xffffffffu, st_envs, o);
-      st_cmax = max(st_cmax, __shfl_down_sync(0xffffffffu, st_cmax, o));
-    }
-    if (lane == 0) {
-      double *slot = stats_partial + (size_t)blockIdx.x * STAT_W;
-      slot[0] += st_r; slot[1] += st_tt; slot[2] += st_bp; slot[3] += st_dup; slot[4] += st_cov;
-      slot[5] = fmax(slot[5], (double)st_cmax);
-      slot[6] += st_envs;
-    }
-  }
+  // warp 0 holds all statistics of the CTA
+  if (warp == 0) stats_commit(stats + (size_t)blockIdx.x * STAT_W, fx_r, fx_tt, fx_bp, fx_dup, st_cov, st_cmax, st_envs);
 }

@@ -265,7 +265,7 @@ __device__ __noinline__ void tile_agent_exact(const ExactK P, const TileMaskPtrs
 template <bool AUX>
 __global__ void __launch_bounds__(TILE_NT, TILE_CTAS_PER_SM)
 uavsim_step_tile_kernel(const KParams P, const UavSimBuffers B, const ActEntry *__restrict__ act_tab, int64_t env_begin,
-                        int64_t env_count, int mode, double coop, int done_flag, double *__restrict__ stats_partial) {
+                        int64_t env_count, int mode, double coop, int done_flag, long long *__restrict__ stats) {
   constexpr int N = 64, M = 64;
   typedef TileSmem<AUX> SmemT;
   static_assert(offsetof(SmemT, bo2) + sizeof(uint4) * 64 - offsetof(SmemT, bt1) >= sizeof(float) * (12 * N + 4 * N), "output staging");
@@ -306,7 +306,7 @@ uavsim_step_tile_kernel(const KParams P, const UavSimBuffers B, const ActEntry *
   const int64_t plane = P.E * N;
   const float inv_dp_f = P.inv_dp_f, inv_dc_f = P.inv_dc_f, inv_na_f = P.inv_na_f;
   const float k_ex0 = 1.4426950408889634f, k_ex1 = P.k_ex1_f;
-  double st_r = 0, st_tt = 0, st_bp = 0, st_dup = 0, st_cov = 0, st_envs = 0;
+  long long fx_r = 0, fx_tt = 0, fx_bp = 0, fx_dup = 0, st_cov = 0, st_envs = 0;  // statistics (common.cuh: sf_fx)
   int st_cmax = 0;
   uint32_t parity = 0;
 
@@ -732,7 +732,7 @@ uavsim_step_tile_kernel(const KParams P, const UavSimBuffers B, const ActEntry *
       s_rew[N + t] = ttn;
       s_rew[2 * N + t] = bpn;
       s_rew[3 * N + t] = dupn;
-      st_tt += (double)ttn; st_bp += (double)bpn; st_dup += (double)dupn;
+      fx_tt += sf_fx(ttn); fx_bp += sf_fx(bpn); fx_dup += sf_fx(dupn);
     }
     if (slow && AUX && B.tracker_cnt) {
       __syncthreads();
@@ -771,7 +771,7 @@ uavsim_step_tile_kernel(const KParams P, const UavSimBuffers B, const ActEntry *
         }
         r = fminf(fmaxf(r, -1.0f), 1.0f);  // clip_and_normalize(reward, -1, 1) is a plain clip
         s_rew[t] = r;
-        if (!pmi_pending) st_r += (double)r;
+        if (!pmi_pending) fx_r += sf_fx(r);
       }
     } else {
       // neighbour mean as one more masked sum: the neighbour bits of column tile J, read as fp16, x {raw hi, 1, raw lo} x scale
@@ -799,7 +799,7 @@ uavsim_step_tile_kernel(const KParams P, const UavSimBuffers B, const ActEntry *
           float r = (cnt > 0.5f) ? fmaf(1.0f - cf, rw, cf * s * sf_rcp(cnt)) : 0.0f;
           r = fminf(fmaxf(r, -1.0f), 1.0f);
           s_rew[row] = r;
-          st_r += (double)r;
+          fx_r += sf_fx(r);
         }
       }
     }
@@ -828,16 +828,14 @@ uavsim_step_tile_kernel(const KParams P, const UavSimBuffers B, const ActEntry *
                     __popc(S.cover[0][1] | S.cover[1][1] | S.cover[2][1] | S.cover[3][1]);
       B.covered[e] = c;
       if (B.done) B.done[e] = done_flag;
-      st_cov += (double)c;
+      st_cov += c;
       st_cmax = max(st_cmax, c);
-      st_envs += 1.0;
+      st_envs++;
     }
   }
   __syncwarp();
   if (warp == 0) {
     if (elect_one()) asm volatile("cp.async.bulk.wait_group 0;" ::: "memory");  // outputs complete before the CTA retires
   }
-  __syncthreads();
-  block_stats_commit(reinterpret_cast<double *>(S.ux), stats_partial + (size_t)blockIdx.x * STAT_W, st_r, st_tt, st_bp,
-                     st_dup, st_cov, st_cmax, st_envs, TILE_NT);
+  stats_commit(stats + (size_t)blockIdx.x * STAT_W, fx_r, fx_tt, fx_bp, fx_dup, st_cov, st_cmax, st_envs);
 }

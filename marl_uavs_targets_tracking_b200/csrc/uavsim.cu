@@ -312,11 +312,10 @@ static int uavsim_create_impl(const UavSimParams *p, int64_t n_envs, int64_t env
   }
   h->stat_slots = h->grid_max > 4096 ? h->grid_max : 4096;
   if (small_warps > h->stat_slots) h->stat_slots = small_warps;  // one statistics slot per CTA of that kernel too
-  h->kp.stat_slots = h->stat_slots;
-  CUDA_TRY(cudaMalloc(&h->d_stats, sizeof(double) * 3 * h->stat_slots * STAT_W));
+  CUDA_TRY(cudaMalloc(&h->d_stats, sizeof(long long) * h->stat_slots * STAT_W));
   CUDA_TRY(cudaMalloc(&h->d_stats8, sizeof(double) * 8));
   CUDA_TRY(cudaMallocHost(&h->h_stats8, sizeof(double) * 8));
-  CUDA_TRY(cudaMemset(h->d_stats, 0, sizeof(double) * 3 * h->stat_slots * STAT_W));
+  CUDA_TRY(cudaMemset(h->d_stats, 0, sizeof(long long) * h->stat_slots * STAT_W));
 
   CUDA_TRY(cudaStreamCreateWithFlags(&h->s_in, cudaStreamNonBlocking));
   CUDA_TRY(cudaStreamCreateWithFlags(&h->s_comp, cudaStreamNonBlocking));
@@ -382,7 +381,7 @@ static int check_bound(uavsim_t *h, const char *who) {
 }
 
 static int clear_counters(uavsim_t *h, cudaStream_t st) {
-  const int count = 3 * h->stat_slots * STAT_W;  // (an all-zero double is an all-zero int64)
+  const int count = h->stat_slots * STAT_W;
   uavsim_stats_clear_kernel<<<(count + 255) / 256, 256, 0, st>>>(h->d_stats, count);
   CUDA_TRY(cudaGetLastError());
   h->launches++;
@@ -468,8 +467,7 @@ static int pmi_launch_t(uavsim_t *h, int64_t e0, int64_t cnt, double coop, cudaS
   }
   const int64_t ngroups = (cnt + h->pmi_g - 1) / h->pmi_g;
   const int grid = (int)(ngroups < h->pmi_grid_max ? ngroups : h->pmi_grid_max);
-  kern<<<grid, PMI_NT, h->smem_pmi, st>>>(h->kp, h->buf, h->pmi, e0, cnt, h->pmi_g, h->pmi_pmax, coop,
-                                         h->d_stats + (size_t)h->stat_slots * STAT_W);
+  kern<<<grid, PMI_NT, h->smem_pmi, st>>>(h->kp, h->buf, h->pmi, e0, cnt, h->pmi_g, h->pmi_pmax, coop, h->d_stats);
   CUDA_TRY(cudaGetLastError());
   h->launches++;
   return 0;
@@ -518,11 +516,9 @@ static int pmi_tc_launch(uavsim_t *h, int64_t e0, int64_t cnt, double coop, cuda
   int grid = (int)(ngroups < h->sm_count ? ngroups : h->sm_count);
   if (grid > h->stat_slots) grid = h->stat_slots;
   if (h->pmi.H == 64)
-    uavsim_pmi_tc_kernel<64><<<grid, TC_NT, TcSmem::total, st>>>(h->kp, h->buf, W, e0, cnt, G, coop,
-                                                                h->d_stats + (size_t)h->stat_slots * STAT_W);
+    uavsim_pmi_tc_kernel<64><<<grid, TC_NT, TcSmem::total, st>>>(h->kp, h->buf, W, e0, cnt, G, coop, h->d_stats);
   else
-    uavsim_pmi_tc_kernel<128><<<grid, TC_NT, TcSmem::total, st>>>(h->kp, h->buf, W, e0, cnt, G, coop,
-                                                                 h->d_stats + (size_t)h->stat_slots * STAT_W);
+    uavsim_pmi_tc_kernel<128><<<grid, TC_NT, TcSmem::total, st>>>(h->kp, h->buf, W, e0, cnt, G, coop, h->d_stats);
   CUDA_TRY(cudaGetLastError());
   h->launches++;
   return 0;
@@ -750,8 +746,7 @@ static int launch_step_range(uavsim_t *h, int mode, double coop, int64_t e0, int
       at[0].val.programmaticStreamSerializationAllowed = 1;
       cfg.attrs = at; cfg.numAttrs = 1;
       const ActEntry *act_c = h->d_act;
-      double *stats_p = h->d_stats;
-      CUDA_TRY(cudaLaunchKernelEx(&cfg, h->small_fn[v], h->kp, h->buf, act_c, e0, cnt, mode, coop, done_flag, stats_p, rng_on, rng_seed, rng_step));
+      CUDA_TRY(cudaLaunchKernelEx(&cfg, h->small_fn[v], h->kp, h->buf, act_c, e0, cnt, mode, coop, done_flag, h->d_stats, rng_on, rng_seed, rng_step));
     } else {
       h->small_fn[v]<<<grid, SMALL_NT, 0, st>>>(h->kp, h->buf, h->d_act, e0, cnt, mode, coop, done_flag, h->d_stats, rng_on, rng_seed, rng_step);
     }

@@ -484,25 +484,64 @@ def test_host_buffer_step_equals_device_step(method, hidden):
     a_env.close(); b_env.close()
 
 
-def test_episode_stats_equal_output_sums():
-    from marl_uavs_targets_tracking_b200 import default_config
-    cfg = default_config("MAAC-G", 10, 10)
-    env = _env(10, 10, cfg, 777, seed=2)
+def _fx_counts(rew4):
+    """The four reward planes as integer counts of 2^-22 (common.cuh: sf_fx), summed per plane."""
+    v = rew4.float().cpu().numpy().reshape(4, -1)
+    fx = (v + np.float32(3.0)).astype(np.float32).view(np.int32).astype(np.int64) - 0x40400000
+    return fx.sum(axis=1)
+
+
+def _check_episode_stats_equal_output_sums(n, method, hidden, step_path, pmi_path, rollout):
+    from marl_uavs_targets_tracking_b200 import PMINetwork, default_config
+    cfg = default_config(method, n, n)
+    torch.manual_seed(0)
+    pmi = PMINetwork(hidden_dim=hidden).eval() if hidden else None
+    E, T = (300, 6) if n == 64 else (777, 20)
+    env = _env(n, n, cfg, E, seed=2)
+    env.set_step_path(step_path)
+    env.set_pmi_path(pmi_path)
     env.reset(cfg)
-    acc = np.zeros(4)
+    fx = np.zeros(4, dtype=np.int64)
     cs, cm = 0, 0
-    for t in range(20):
-        env.random_actions(1, t)
-        _, rew4, cov = env.step_device(cfg, None)
-        acc += rew4.double().sum(dim=(1, 2)).cpu().numpy()
+    for t in range(T):
+        if rollout:
+            _, rew4, cov = env.run_random_policy(cfg, pmi, 1, t, 1)
+        else:
+            env.random_actions(1, t)
+            _, rew4, cov = env.step_device(cfg, pmi)
+        fx += _fx_counts(rew4)
         cs += int(cov.sum()); cm = max(cm, int(cov.max()))
     s = env.episode_stats()
-    got = np.array([s["rewards"], s["target_tracking_reward"], s["boundary_punishment"], s["duplicate_tracking_punishment"]])
-    np.testing.assert_allclose(got, acc, rtol=1e-6, atol=1e-3)  # outputs are fp32, the accumulators fp64
-    assert s["covered_sum"] == cs and s["covered_max"] == cm and s["env_steps"] == 777 * 20
+    got = [s["rewards"], s["target_tracking_reward"], s["boundary_punishment"], s["duplicate_tracking_punishment"]]
+    assert got == [float(c) * 2.0 ** -22 for c in fx]
+    assert s["covered_sum"] == cs and s["covered_max"] == cm and s["env_steps"] == E * T
+    assert s["pmi_rows_out_of_range"] == 0
     env.reset(cfg)
     assert env.episode_stats()["env_steps"] == 0
     env.close()
+
+
+def test_episode_stats_equal_output_sums():
+    """episode_stats() is exactly what the steps wrote: the four reward sums are the integer sums of the float32 outputs
+    as counts of 2^-22 (times 2^-22), covered sum / max and env-steps are equal (10x10, automatic kernel choice)."""
+    _check_episode_stats_equal_output_sums(10, "MAAC-G", 0, 0, 0, False)
+
+
+@pytest.mark.parametrize("n,method,hidden,step_path,pmi_path,rollout", [
+    pytest.param(64, "MAAC-G", 0, 1, 0, False, id="64x64-generic"),
+    pytest.param(64, "MAAC-G", 0, 2, 0, False, id="64x64-fast"),
+    pytest.param(64, "MAAC-G", 0, 3, 0, False, id="64x64-tile"),
+    pytest.param(10, "MAAC-G", 0, 1, 0, False, id="10x10-generic"),
+    pytest.param(10, "MAAC-G", 0, 4, 0, False, id="10x10-small"),
+    pytest.param(10, "MAAC-G", 0, 0, 0, True, id="10x10-rollout"),
+    pytest.param(10, "MAAC-R", 32, 0, 0, False, id="10x10-pmi-cuda-cores-h32"),
+    pytest.param(10, "MAAC-R", 64, 0, 1, False, id="10x10-pmi-cuda-cores-h64"),
+    pytest.param(10, "MAAC-R", 128, 0, 0, False, id="10x10-pmi-tensor-h128"),
+])
+def test_episode_stats_equal_output_sums_on_every_path(n, method, hidden, step_path, pmi_path, rollout):
+    """The same exact equality whichever kernel served the steps: every step kernel, the rollout loop below the FFI and
+    both PMI kernels keep their statistics in one fixed-point format."""
+    _check_episode_stats_equal_output_sums(n, method, hidden, step_path, pmi_path, rollout)
 
 
 def test_reference_shaped_api_single_env():
