@@ -244,6 +244,34 @@ typedef struct {
 int uavsim_policy_sample(const float *obs, int64_t rows, const UavSimPolicyWeights *w, uint64_t seed, uint64_t counter,
                          int32_t *actions, float *probs, int device, void *stream);
 
+/* Device trajectory buffers of uavsim_run_policy (T = nsteps); any field may be NULL: that output then goes to the
+ * bound buffer, overwritten step by step.  obs must be 16-byte aligned, like the bound observation buffer. */
+typedef struct UavSimTrajectory {
+  float *obs;        /* [T+1,E,n,12]: slot 0 <- the bound observation before the first step, slot k+1 <- step k */
+  int32_t *actions;  /* [T,E,n]     : the actions drawn for step k */
+  float *rew4;       /* [T,4,E,n]   : the four reward planes of step k */
+  int32_t *covered;  /* [T,E]       : covered targets after step k */
+} UavSimTrajectory;
+
+/* Learned-policy rollout of a whole episode without returning to the caller between steps (src/train.py:160-176 for
+ * all environments at once): for k = 0 .. nsteps-1
+ *     uavsim_policy_sample(obs_k, E*n, w, seed, first_counter + k, actions_k, NULL, device, stream);
+ *     uavsim_step(h, mode, cooperative, stream);
+ * where obs_k / actions_k (and the step's obs / rew4 / covered outputs) are the trajectory slots of step k, or the bound
+ * buffers where a field of `traj` is NULL (traj may be NULL: everything in place).  The result is bit-identical to that
+ * loop in every output -- observations, actions, reward planes, covered counts, done, the state, the step counter and
+ * uavsim_episode_stats -- because the same kernels run on the same data: the step kernel is chosen as uavsim_step chooses
+ * it.  The policy launches and the small-swarm step kernel use programmatic dependent launch, so each grid is scheduled
+ * while its predecessor drains (the policy kernel stages its weights meanwhile).  After the last step the last slot of
+ * every given field is copied into the bound buffer, so the bound obs / actions / rew4 / covered hold what stepping one
+ * step at a time leaves there, and the next uavsim_step continues the episode.  The bound pointers are restored on
+ * every exit.  Every argument is checked before anything is queued: on an error nothing is enqueued and the step
+ * counter does not move (n_actions must equal the handle's na; with uavsim_set_step_path 2 or 3 every trajectory slot
+ * must be 16-byte aligned, i.e. E*n % 4 == 0 when actions are recorded, else UAVSIM_ERR_UNSUPPORTED).  The policy
+ * launches count in uavsim_launch_count. */
+int uavsim_run_policy(uavsim_t *h, int mode, double cooperative, const UavSimPolicyWeights *w, uint64_t seed,
+                      uint64_t first_counter, int64_t nsteps, const UavSimTrajectory *traj, void *stream);
+
 #ifdef __cplusplus
 }
 #endif

@@ -38,6 +38,10 @@ class UavSimPolicyWeights(C.Structure):
                 ("w1", C.c_void_p), ("b1", C.c_void_p), ("w2", C.c_void_p), ("b2", C.c_void_p)]
 
 
+class UavSimTrajectory(C.Structure):
+    _fields_ = [(k, C.c_void_p) for k in ("obs", "actions", "rew4", "covered")]
+
+
 class UavSimPmiWeights(C.Structure):
     _fields_ = [("hidden", C.c_int32), ("_pad", C.c_int32), ("w0", C.c_void_p), ("b0", C.c_void_p),
                 ("w1", C.c_void_p), ("b1", C.c_void_p), ("w2", C.c_void_p), ("b2", C.c_float), ("_pad2", C.c_float)]
@@ -70,6 +74,8 @@ SYMBOLS = {
     "uavsim_step_count": (C.c_int64, [_H]),
     "uavsim_policy_sample": (C.c_int, [C.c_void_p, C.c_int64, C.POINTER(UavSimPolicyWeights), C.c_uint64, C.c_uint64,
                                        C.c_void_p, C.c_void_p, C.c_int, C.c_void_p]),
+    "uavsim_run_policy": (C.c_int, [_H, C.c_int, C.c_double, C.POINTER(UavSimPolicyWeights), C.c_uint64, C.c_uint64,
+                                    C.c_int64, C.POINTER(UavSimTrajectory), C.c_void_p]),
     # prioritized replay (src/train.py:73-139)
     "uavsim_replay_create": (C.c_int, [C.c_int64, C.c_int, C.c_double, C.c_int, C.POINTER(_H)]),
     "uavsim_replay_destroy": (C.c_int, [_H]),

@@ -42,7 +42,10 @@ __device__ __forceinline__ float pol_hi(uint64_t v) { return __uint_as_float((ui
 //   [ 0..23]  {w1[j][k], w1[j+1][k]} for k = 0..11        [24..25] {b1[j], b1[j+1]}   [26..31] 0
 //   [32..63]  {w2[a][j], w2[a][j+1]} for a = 0..AP-1 (0 beyond the action count)
 // AP = number of actions rounded up to a multiple of 4; the padding logits are -inf (probability 0)
-template <int AP>
+// PDL: the form uavsim_run_policy launches with programmatic dependent launch.  The weights are constant for the whole
+// call, so they are staged before griddepcontrol.wait and that overlaps the previous step kernel's tail; nothing else
+// touches global memory before the wait.  Launched without the attribute, the wait passes straight through.
+template <int AP, bool PDL = false>
 __global__ void __launch_bounds__(POLICY_NT)
 uavsim_policy_kernel(const float *__restrict__ obs, int64_t rows, const PolicyDev W, uint64_t seed, uint64_t counter,
                      int32_t *__restrict__ actions, float *__restrict__ probs) {
@@ -59,6 +62,10 @@ uavsim_policy_kernel(const float *__restrict__ obs, int64_t rows, const PolicyDe
     s_w[k] = v;
   }
   __syncthreads();
+  if (PDL) {
+    asm volatile("griddepcontrol.wait;" ::: "memory");
+    asm volatile("griddepcontrol.launch_dependents;" ::: "memory");
+  }
 
   const int64_t stride = (int64_t)gridDim.x * POLICY_NT * POLICY_ROWS;
   for (int64_t r0 = ((int64_t)blockIdx.x * POLICY_NT + threadIdx.x) * POLICY_ROWS; r0 < rows; r0 += stride) {
@@ -133,15 +140,46 @@ uavsim_policy_kernel(const float *__restrict__ obs, int64_t rows, const PolicyDe
 // ------------------------------------------------------------------------------------------------
 // host side
 // ------------------------------------------------------------------------------------------------
-template <int AP>
-static int policy_launch(const float *obs, int64_t rows, const PolicyDev &W, uint64_t seed, uint64_t counter,
-                         int32_t *actions, float *probs, int device, cudaStream_t st) {
-  const size_t smem = (size_t)((W.H + 1) / 2) * 64 * sizeof(float);
-  int rc = raise_dynamic_smem((const void *)uavsim_policy_kernel<AP>, device, smem);
+typedef void (*PolicyKernelFn)(const float *, int64_t, const PolicyDev, uint64_t, uint64_t, int32_t *, float *);
+
+// One policy launch over `rows` rows: the kernel instance, its dynamic shared memory and grid.
+struct PolicyLaunch {
+  PolicyKernelFn fn;
+  size_t smem;
+  int blocks;
+};
+
+// The weight rules of the fused policy kernel (shared by uavsim_policy_sample and uavsim_run_policy).
+static int policy_check_weights(const UavSimPolicyWeights *w, const char *who) {
+  if (!w || !w->w1 || !w->b1 || !w->w2 || !w->b2) { SET_ERR("%s: NULL argument", who); return UAVSIM_ERR_ARG; }
+  if (w->state_dim != POLICY_IN || w->hidden < 1 || w->hidden > POLICY_HMAX || w->n_actions < 2 || w->n_actions > POLICY_AMAX) {
+    SET_ERR("%s: supports state_dim = %d, hidden <= %d, 2 <= n_actions <= %d (got %d, %d, %d)", who, POLICY_IN,
+            POLICY_HMAX, POLICY_AMAX, w->state_dim, w->hidden, w->n_actions);
+    return UAVSIM_ERR_UNSUPPORTED;
+  }
+  return 0;
+}
+
+static PolicyDev policy_dev(const UavSimPolicyWeights *w) {
+  PolicyDev W;
+  W.w1 = w->w1; W.b1 = w->b1; W.w2 = w->w2; W.b2 = w->b2; W.H = w->hidden; W.A = w->n_actions;
+  return W;
+}
+
+// (weights already checked by policy_check_weights; needs the current device set)
+static int policy_plan(int64_t rows, const PolicyDev &W, bool pdl, int device, PolicyLaunch *L) {
+  switch ((W.A + 3) / 4) {
+    case 1: L->fn = pdl ? uavsim_policy_kernel<4, true> : uavsim_policy_kernel<4>; break;
+    case 2: L->fn = pdl ? uavsim_policy_kernel<8, true> : uavsim_policy_kernel<8>; break;
+    case 3: L->fn = pdl ? uavsim_policy_kernel<12, true> : uavsim_policy_kernel<12>; break;
+    default: L->fn = pdl ? uavsim_policy_kernel<16, true> : uavsim_policy_kernel<16>; break;
+  }
+  L->smem = (size_t)((W.H + 1) / 2) * 64 * sizeof(float);
+  int rc = raise_dynamic_smem((const void *)L->fn, device, L->smem);
   if (rc) return rc;
   int sms = 148, occ = 1;
   cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, device);
-  cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, uavsim_policy_kernel<AP>, POLICY_NT, smem);
+  cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, L->fn, POLICY_NT, L->smem);
   if (occ < 1) occ = 1;
   // persistent, balanced grid: every CTA stages the weights once and runs the same number of 512-row iterations
   // (a grid of "one CTA per iteration" pays the staging per iteration and ends in a mostly idle last wave)
@@ -149,33 +187,25 @@ static int policy_launch(const float *obs, int64_t rows, const PolicyDev &W, uin
   const int64_t resident = (int64_t)sms * occ;
   const int64_t per_cta = (iters + resident - 1) / resident;
   int64_t blocks = (iters + per_cta - 1) / (per_cta > 0 ? per_cta : 1);
-  if (blocks < 1) blocks = 1;
-  uavsim_policy_kernel<AP><<<(int)blocks, POLICY_NT, smem, st>>>(obs, rows, W, seed, counter, actions, probs);
-  CUDA_TRY(cudaGetLastError());
+  L->blocks = (int)(blocks < 1 ? 1 : blocks);
   return 0;
 }
 
 extern "C" int uavsim_policy_sample(const float *obs, int64_t rows, const UavSimPolicyWeights *w, uint64_t seed,
                                     uint64_t counter, int32_t *actions, float *probs, int device, void *stream) {
-  if (!w || rows < 0 || (rows > 0 && (!obs || !actions)) || !w->w1 || !w->b1 || !w->w2 || !w->b2) {
+  if (!w || rows < 0 || (rows > 0 && (!obs || !actions))) {
     SET_ERR("uavsim_policy_sample: NULL argument");
     return UAVSIM_ERR_ARG;
   }
-  if (w->state_dim != POLICY_IN || w->hidden < 1 || w->hidden > POLICY_HMAX || w->n_actions < 2 || w->n_actions > POLICY_AMAX) {
-    SET_ERR("uavsim_policy_sample: supports state_dim = %d, hidden <= %d, 2 <= n_actions <= %d (got %d, %d, %d)", POLICY_IN,
-            POLICY_HMAX, POLICY_AMAX, w->state_dim, w->hidden, w->n_actions);
-    return UAVSIM_ERR_UNSUPPORTED;
-  }
+  int rc = policy_check_weights(w, "uavsim_policy_sample");
+  if (rc) return rc;
   if (rows == 0) return 0;
   CUDA_TRY(cudaSetDevice(device));
-  PolicyDev W;
-  W.w1 = w->w1; W.b1 = w->b1; W.w2 = w->w2; W.b2 = w->b2; W.H = w->hidden; W.A = w->n_actions;
-  cudaStream_t st = (cudaStream_t)stream;
-  switch ((w->n_actions + 3) / 4) {
-    case 1: return policy_launch<4>(obs, rows, W, seed, counter, actions, probs, device, st);
-    case 2: return policy_launch<8>(obs, rows, W, seed, counter, actions, probs, device, st);
-    case 3: return policy_launch<12>(obs, rows, W, seed, counter, actions, probs, device, st);
-    case 4: return policy_launch<16>(obs, rows, W, seed, counter, actions, probs, device, st);
-  }
-  return UAVSIM_ERR_UNSUPPORTED;
+  const PolicyDev W = policy_dev(w);
+  PolicyLaunch L;
+  rc = policy_plan(rows, W, false, device, &L);
+  if (rc) return rc;
+  L.fn<<<L.blocks, POLICY_NT, L.smem, (cudaStream_t)stream>>>(obs, rows, W, seed, counter, actions, probs);
+  CUDA_TRY(cudaGetLastError());
+  return 0;
 }

@@ -524,16 +524,27 @@ static int pmi_tc_launch(uavsim_t *h, int64_t e0, int64_t cnt, double coop, cuda
   return 0;
 }
 
-static int pmi_launch(uavsim_t *h, int64_t e0, int64_t cnt, double coop, cudaStream_t st, bool configure_only) {
-  if (!configure_only && pmi_use_tensor(h)) return pmi_tc_launch(h, e0, cnt, coop, st);
-  if (!configure_only && h->pmi_path == 2) {  // (weights uploaded after the path was chosen)
+// Whether a PMI kernel can serve the uploaded weights with the selected path (checked again at every launch: weights
+// may be uploaded after the path was chosen).
+static int pmi_servable(const uavsim_t *h) {
+  if (pmi_use_tensor(h)) return 0;
+  if (h->pmi_path == 2) {
     SET_ERR("PMI mode: tensor-core path selected (uavsim_set_pmi_path 2) but unavailable: %s", pmi_tensor_why_not(h));
     return UAVSIM_ERR_UNSUPPORTED;
   }
-  if (!configure_only && !h->has_cc) {
+  if (!h->has_cc) {
     SET_ERR("PMI mode: n_uav=%d is too large for the CUDA-core PMI kernel and the tensor path is %s", h->kp.n,
             h->pmi_path == 1 ? "switched off (uavsim_set_pmi_path 1)" : "unavailable (hidden is neither 64 nor 128)");
     return UAVSIM_ERR_UNSUPPORTED;
+  }
+  return 0;
+}
+
+static int pmi_launch(uavsim_t *h, int64_t e0, int64_t cnt, double coop, cudaStream_t st, bool configure_only) {
+  if (!configure_only && pmi_use_tensor(h)) return pmi_tc_launch(h, e0, cnt, coop, st);
+  if (!configure_only) {
+    const int rc = pmi_servable(h);
+    if (rc) return rc;
   }
   switch (h->pmi.H) {
     case 32: return pmi_launch_t<2, 64>(h, e0, cnt, coop, st, configure_only);
@@ -731,14 +742,16 @@ static bool small_path_in_use(const uavsim_t *h, int64_t cnt, bool rollout = fal
   const int64_t waves2 = rollout ? 20 : 5;  // twice the number of waves
   return (cnt + G - 1) / G <= (int64_t)h->small_grid_max[0] * waves2 / 2;
 }
+// `pdl`: a rollout loop below the FFI -- the small-swarm kernel is launched with programmatic dependent launch (the
+// other step kernels and the PMI kernels launch plainly).
 static int launch_step_range(uavsim_t *h, int mode, double coop, int64_t e0, int64_t cnt, int done_flag, cudaStream_t st,
-                             int rng_on = 0, uint64_t rng_seed = 0, uint32_t rng_step = 0) {
+                             bool pdl = false, int rng_on = 0, uint64_t rng_seed = 0, uint32_t rng_step = 0) {
   if (small_path_in_use(h, cnt, rng_on != 0)) {  // groups of environments in two-warp CTAs
     const int v = (h->buf.obs_mask || h->buf.tracker_cnt) ? 1 : 0;
     const int G = small_group(h->kp.n, h->kp.m);
     const int64_t groups = (cnt + G - 1) / G;
     const int grid = (int)(groups < h->small_grid_max[v] ? groups : h->small_grid_max[v]);
-    if (rng_on) {  // a rollout loop: let this grid be scheduled while the previous step drains (it waits before its first load)
+    if (pdl) {  // let this grid be scheduled while the previous kernel drains (it waits before its first load)
       cudaLaunchConfig_t cfg = {};
       cfg.gridDim = dim3((unsigned)grid); cfg.blockDim = dim3(SMALL_NT); cfg.dynamicSmemBytes = 0; cfg.stream = st;
       cudaLaunchAttribute at[1];
@@ -804,7 +817,7 @@ extern "C" int uavsim_run_random_policy(uavsim_t *h, int mode, double coop, uint
       CUDA_TRY(cudaSetDevice(h->device));
       h->t++;
       const int done = (h->hp.num_steps > 0 && h->t >= h->hp.num_steps) ? 1 : 0;
-      rc = launch_step_range(h, mode, coop, 0, h->E, done, (cudaStream_t)stream, 1, seed, (uint32_t)(first_step + k));
+      rc = launch_step_range(h, mode, coop, 0, h->E, done, (cudaStream_t)stream, true, 1, seed, (uint32_t)(first_step + k));
       if (rc) return rc;
       continue;
     }
@@ -813,6 +826,83 @@ extern "C" int uavsim_run_random_policy(uavsim_t *h, int mode, double coop, uint
     rc = uavsim_step(h, mode, coop, stream);
     if (rc) return rc;
   }
+  return 0;
+}
+
+// Learned-policy rollout below the FFI: nsteps x (policy launch, step) queued back to back.  The handle's bound
+// obs / actions / rew4 / covered pointers are pointed at the trajectory slots of each step (the kernels take the buffer
+// struct by value, so this costs nothing) and restored before returning.  The step kernel is chosen exactly as
+// uavsim_step chooses it -- not with the wider small-kernel range of the random-policy loop, whose draw is fused into
+// that kernel -- so every output is bit-identical to the per-step calls.
+extern "C" int uavsim_run_policy(uavsim_t *h, int mode, double coop, const UavSimPolicyWeights *w, uint64_t seed,
+                                 uint64_t first_counter, int64_t nsteps, const UavSimTrajectory *traj, void *stream) {
+  const char *who = "uavsim_run_policy";
+  int rc = check_step_args(h, mode, coop, who);
+  if (rc) return rc;
+  if (nsteps < 0) { SET_ERR("%s: nsteps < 0", who); return UAVSIM_ERR_ARG; }
+  rc = policy_check_weights(w, who);
+  if (rc) return rc;
+  if (w->n_actions != h->kp.na) { SET_ERR("%s: the policy has %d actions, the environment na = %d", who, w->n_actions, h->kp.na); return UAVSIM_ERR_ARG; }
+  const UavSimTrajectory tr = traj ? *traj : UavSimTrajectory{nullptr, nullptr, nullptr, nullptr};
+  if ((reinterpret_cast<uintptr_t>(tr.obs) & 15) != 0) { SET_ERR("%s: trajectory obs must be 16-byte aligned", who); return UAVSIM_ERR_ARG; }
+  const UavSimBuffers home = h->buf;
+  const int64_t E = h->E, en = E * h->kp.n;
+  auto bind_slot = [&](int64_t k) {
+    h->buf.obs = tr.obs ? tr.obs + (k + 1) * en * 12 : home.obs;
+    h->buf.actions = tr.actions ? tr.actions + k * en : home.actions;
+    h->buf.rew4 = tr.rew4 ? tr.rew4 + k * 4 * en : home.rew4;
+    h->buf.covered = tr.covered ? tr.covered + k * E : home.covered;
+  };
+  if (h->step_path == 2 || h->step_path == 3) {  // the 64 x 64 kernels need every array 16-byte aligned
+    bool ok = true;
+    for (int64_t k = 0; k < nsteps && k < 4; k++) {  // (slot offsets are multiples of 4 bytes: alignment repeats after 4)
+      bind_slot(k);
+      ok = ok && fast_path_usable(h);
+    }
+    h->buf = home;
+    if (!ok) {
+      SET_ERR("%s: the selected step kernel needs 16-byte aligned trajectory slots (E*n %% 4 == 0 for actions)", who);
+      return UAVSIM_ERR_UNSUPPORTED;
+    }
+  }
+  if (mode == UAVSIM_MODE_PMI && coop != 0.0) {
+    rc = pmi_servable(h);
+    if (rc) return rc;
+  }
+  CUDA_TRY(cudaSetDevice(h->device));
+  const PolicyDev W = policy_dev(w);
+  PolicyLaunch L;
+  rc = policy_plan(en, W, true, h->device, &L);
+  if (rc) return rc;
+
+  cudaStream_t st = (cudaStream_t)stream;
+  if (tr.obs) CUDA_TRY(cudaMemcpyAsync(tr.obs, home.obs, sizeof(float) * en * 12, cudaMemcpyDeviceToDevice, st));
+  for (int64_t k = 0; k < nsteps && rc == 0; k++) {
+    const float *obs_k = tr.obs ? tr.obs + k * en * 12 : home.obs;
+    bind_slot(k);
+    // The first policy launch follows the caller's own work (which may have just written the weights): a plain launch.
+    // Later ones follow this loop's step or PMI kernel and may start early.
+    cudaLaunchConfig_t cfg = {};
+    cfg.gridDim = dim3((unsigned)L.blocks); cfg.blockDim = dim3(POLICY_NT); cfg.dynamicSmemBytes = L.smem; cfg.stream = st;
+    cudaLaunchAttribute at[1];
+    at[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
+    at[0].val.programmaticStreamSerializationAllowed = k > 0 ? 1 : 0;
+    cfg.attrs = at; cfg.numAttrs = 1;
+    float *no_probs = nullptr;
+    cudaError_t e = cudaLaunchKernelEx(&cfg, L.fn, obs_k, en, W, seed, first_counter + (uint64_t)k, h->buf.actions, no_probs);
+    if (e != cudaSuccess) { SET_ERR("%s: policy launch failed: %s", who, cudaGetErrorString(e)); rc = (int)e; break; }
+    h->launches++;
+    h->t++;
+    const int done = (h->hp.num_steps > 0 && h->t >= h->hp.num_steps) ? 1 : 0;
+    rc = launch_step_range(h, mode, coop, 0, E, done, st, true);
+  }
+  h->buf = home;
+  if (rc || nsteps == 0) return rc;
+  // the bound buffers end as the per-step calls leave them: the last step's outputs and actions
+  if (tr.obs) CUDA_TRY(cudaMemcpyAsync(home.obs, tr.obs + nsteps * en * 12, sizeof(float) * en * 12, cudaMemcpyDeviceToDevice, st));
+  if (tr.actions) CUDA_TRY(cudaMemcpyAsync(home.actions, tr.actions + (nsteps - 1) * en, sizeof(int32_t) * en, cudaMemcpyDeviceToDevice, st));
+  if (tr.rew4) CUDA_TRY(cudaMemcpyAsync(home.rew4, tr.rew4 + (nsteps - 1) * 4 * en, sizeof(float) * 4 * en, cudaMemcpyDeviceToDevice, st));
+  if (tr.covered) CUDA_TRY(cudaMemcpyAsync(home.covered, tr.covered + (nsteps - 1) * E, sizeof(int32_t) * E, cudaMemcpyDeviceToDevice, st));
   return 0;
 }
 

@@ -20,8 +20,10 @@ import numpy as np
 import torch
 
 from . import _cabi
-from ._cabi import MODE_MEAN, MODE_PMI, MODE_SELF, UavSimBuffers, UavSimError, UavSimParams, UavSimPmiWeights
+from ._cabi import (MODE_MEAN, MODE_PMI, MODE_SELF, UavSimBuffers, UavSimError, UavSimParams, UavSimPmiWeights,
+                    UavSimTrajectory)
 from .pmi import fold_pmi, pmi_version
+from .rollout import policy_weights
 
 _REWARD_KEYS = ("rewards", "target_tracking_reward", "boundary_punishment", "duplicate_tracking_punishment")
 
@@ -300,6 +302,41 @@ class BatchedEnvironment:
         with self._on_device():
             _cabi.check(self._lib.uavsim_run_random_policy(self._h, mode, coop, C.c_uint64(seed), int(first_step),
                                                            int(nsteps), self._stream()), "uavsim_run_random_policy")
+        self._host = None
+        return self._obs, self._rew4, self._covered
+
+    def run_policy(self, config, pmi, policy, seed, first_counter, nsteps, obs=None, actions=None, rew4=None,
+                   covered=None):
+        """`nsteps` steps of a learned policy queued from C without returning to Python in between
+        (uavsim_run_policy).  `policy` is a PolicyNet (or a DDP wrapper around one) on this device; step k draws its
+        actions with the fused policy kernel, counter `first_counter + k`, exactly what `fused_policy_sample(policy,
+        states, seed, first_counter + k, out=actions)` followed by `step_device` gives -- bit for bit, in every output.
+
+        Optional trajectory tensors (contiguous, on this device), T = nsteps: obs float32 [T+1,E,n,12] (slot 0 <- the
+        current observation, slot k+1 <- step k), actions int32 [T,E,n], rew4 float32 [T,4,E,n], covered int32 [T,E].
+        A field left None goes to the bound buffer.  Afterwards the bound buffers hold the last step's values, as after
+        stepping one step at a time.  Returns the bound (obs, rew4, covered)."""
+        if self._h is None:
+            raise UavSimError("step before reset")
+        E, n, T = self.n_envs, self.n_uav, int(nsteps)
+        traj = UavSimTrajectory()
+        for name, t, dtype, shape in (("obs", obs, torch.float32, (T + 1, E, n, 12)),
+                                      ("actions", actions, torch.int32, (T, E, n)),
+                                      ("rew4", rew4, torch.float32, (T, 4, E, n)),
+                                      ("covered", covered, torch.int32, (T, E))):
+            if t is None:
+                continue
+            if t.dtype != dtype or tuple(t.shape) != shape or not t.is_contiguous() or t.device != self.device:
+                raise ValueError("run_policy: %s must be a contiguous %s tensor of shape %s on %s (got %s %s on %s)"
+                                 % (name, dtype, shape, self.device, t.dtype, tuple(t.shape), t.device))
+            setattr(traj, name, t.data_ptr())
+        w, params = policy_weights(policy, self.state_dim)  # (params: kept alive over the call)
+        self._sync_weights(config)
+        mode, coop = self._mode(config, pmi)
+        with self._on_device():
+            _cabi.check(self._lib.uavsim_run_policy(self._h, mode, coop, C.byref(w), C.c_uint64(seed),
+                                                    C.c_uint64(first_counter), T, C.byref(traj), self._stream()),
+                        "uavsim_run_policy")
         self._host = None
         return self._obs, self._rew4, self._covered
 

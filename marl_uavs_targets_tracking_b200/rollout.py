@@ -41,22 +41,29 @@ class ValueNet(nn.Module):
         return self.fc2(F.relu(self.fc1(x))).squeeze(1)
 
 
+def policy_weights(policy, state_dim):
+    """The UavSimPolicyWeights of a PolicyNet (or a DDP wrapper around one) and the tensors it points into, which the
+    caller keeps alive while the struct is in use."""
+    net = policy.module if hasattr(policy, "module") else policy
+    w = _cabi.UavSimPolicyWeights()
+    w.state_dim, w.hidden, w.n_actions = state_dim, net.fc1.out_features, net.fc2.out_features
+    params = [net.fc1.weight, net.fc1.bias, net.fc2.weight, net.fc2.bias]
+    params = [p.detach() if p.is_contiguous() else p.detach().contiguous() for p in params]
+    w.w1, w.b1, w.w2, w.b2 = (p.data_ptr() for p in params)
+    return w, params
+
+
 def fused_policy_sample(policy, states, seed, counter, want_probs=False, out=None):
     """One launch of libuavsim's fused policy kernel (`uavsim_policy_sample`, csrc/policy.cuh): softmax(fc2(relu(fc1(x))))
     and one categorical draw per row, uniforms from Philox4x32-10 keyed (seed; row, counter).  `policy` is a PolicyNet
     (or a DDP wrapper around one) on the device of `states` [B,12] float32; `out` = a contiguous int32 [B] tensor to write
     the actions into (e.g. the environment's bound action buffer).  Returns (actions int32 [B], probs or None)."""
-    net = policy.module if hasattr(policy, "module") else policy
     x = states if (states.dtype == torch.float32 and states.is_contiguous()) else states.float().contiguous()
     dev = x.device
     if dev.type != "cuda":
         raise _cabi.UavSimError("fused_policy_sample needs CUDA tensors (no CPU fallback)")
-    B, H, A = x.shape[0], net.fc1.out_features, net.fc2.out_features
-    w = _cabi.UavSimPolicyWeights()
-    w.state_dim, w.hidden, w.n_actions = x.shape[1], H, A
-    params = [net.fc1.weight, net.fc1.bias, net.fc2.weight, net.fc2.bias]
-    params = [p.detach() if p.is_contiguous() else p.detach().contiguous() for p in params]
-    w.w1, w.b1, w.w2, w.b2 = (p.data_ptr() for p in params)
+    w, params = policy_weights(policy, x.shape[1])
+    B, A = x.shape[0], w.n_actions
     if out is not None:
         assert out.dtype == torch.int32 and out.is_contiguous() and out.numel() == B and out.device == dev
     actions = out if out is not None else torch.empty(B, dtype=torch.int32, device=dev)
@@ -154,14 +161,37 @@ def operate_epoch_batched(config, env, agent, pmi, num_steps, keep_transitions=T
     rewards [T*E*n], next_states [T*E*n,12] (None if keep_transitions is False); summary = the six scalars the
     reference logs per episode, averaged over every environment of every rank.
 
-    With keep_transitions the observations of the whole episode live in ONE [T+1,E,n,12] tensor: the environment's
-    observation buffer is re-bound to slot t+1 before step t, so `states` and `next_states` are overlapping views of it
-    and no observation is copied; the fused policy kernel writes the actions into slot t of the action trajectory,
-    which is bound as the environment's action buffer."""
+    With keep_transitions the observations of the whole episode live in ONE [T+1,E,n,12] tensor: step t writes its
+    observations into slot t+1, so `states` and `next_states` are overlapping views of it and no observation is copied;
+    the actions of step t go to slot t of an [T,E,n] action trajectory.
+
+    With the fused policy (agent.fused) the whole episode is one library call, `env.run_policy` (uavsim_run_policy):
+    the per-step interpreter and FFI time is gone, and the result is bit-identical to driving the steps from Python
+    (step t draws with counter agent._calls + 1 + t, as take_actions would).  With keep_transitions it records all four
+    reward planes of every step, [T,4,E,n] float32: 12 B per agent-step more than the plane-0 buffer of the per-step
+    loop (1.6 GB at 65 536 environments x 10 UAVs x 200 steps).  `rewards` is a copy of plane 0 (4 B per agent-step,
+    allocated while the four planes still exist); the four planes are freed on return.  The stock torch policy
+    (fused=False) is driven step by step from Python."""
     E, n = env.n_envs, env.n_uav
     dev = env.device
     fused = bool(getattr(agent, "fused", False))
-    if keep_transitions:
+    if fused:
+        first_counter = agent._calls + 1
+        if keep_transitions:
+            traj = torch.empty((num_steps + 1, E, n, 12), dtype=torch.float32, device=dev)
+            acts = torch.empty((num_steps, E, n), dtype=torch.int32, device=dev)
+            rew4 = torch.empty((num_steps, 4, E, n), dtype=torch.float32, device=dev)
+            env.run_policy(config, pmi, agent.actor, agent.seed, first_counter, num_steps, obs=traj, actions=acts,
+                           rew4=rew4)
+            transitions = {"states": traj[:-1].reshape(num_steps * E * n, 12), "actions": acts.reshape(-1),
+                           "rewards": rew4[:, 0].reshape(-1), "next_states": traj[1:].reshape(num_steps * E * n, 12)}
+        else:
+            env.run_policy(config, pmi, agent.actor, agent.seed, first_counter, num_steps)
+            transitions = None
+        agent._calls += num_steps
+        if num_steps > 0:
+            config["step"] = num_steps
+    elif keep_transitions:
         home_obs, home_act = env._obs, env.actions
         traj = torch.empty((num_steps + 1, E, n, 12), dtype=torch.float32, device=dev)
         acts = torch.empty((num_steps, E, n), dtype=torch.int32, device=dev)
@@ -172,12 +202,8 @@ def operate_epoch_batched(config, env, agent, pmi, num_steps, keep_transitions=T
                 config["step"] = step + 1
                 env.bind_obs(traj[step + 1])
                 env.bind_actions(acts[step])
-                states = traj[step].view(E * n, 12)
-                if fused:
-                    agent.take_actions(states, out=acts[step].view(-1))
-                else:
-                    a, _ = agent.take_actions(states)
-                    acts[step].view(-1).copy_(a)
+                a, _ = agent.take_actions(traj[step].view(E * n, 12))
+                acts[step].view(-1).copy_(a)
                 _, rew4, _ = env.step_device(config, pmi)
                 rews[step].copy_(rew4[0].reshape(E * n))
         finally:
@@ -189,13 +215,8 @@ def operate_epoch_batched(config, env, agent, pmi, num_steps, keep_transitions=T
     else:
         for step in range(num_steps):
             config["step"] = step + 1
-            states = env._obs.view(E * n, 12)
-            if fused:
-                agent.take_actions(states, out=env.actions.view(-1))
-                env.step_device(config, pmi)
-            else:
-                a, _ = agent.take_actions(states)
-                env.step_device(config, pmi, a.view(E, n))
+            a, _ = agent.take_actions(env._obs.view(E * n, 12))
+            env.step_device(config, pmi, a.view(E, n))
         transitions = None
     stats = reduce_episode_stats(env.episode_stats(), device=env.device)
     return transitions, episode_summary(stats, n)
