@@ -240,7 +240,8 @@ typedef struct {
 } UavSimPolicyWeights;
 
 /* actions[r] ~ Categorical(probs[r, :]) with the uniform Philox4x32-10 (seed; r, counter); probs [rows, n_actions] may be
- * NULL.  obs [rows, 12] float32 (e.g. the environment's observation buffer). */
+ * NULL.  obs [rows, 12] float32 (e.g. the environment's observation buffer), 16-byte aligned: the kernel reads rows with
+ * 16-byte loads, and a misaligned obs is refused with UAVSIM_ERR_ARG. */
 int uavsim_policy_sample(const float *obs, int64_t rows, const UavSimPolicyWeights *w, uint64_t seed, uint64_t counter,
                          int32_t *actions, float *probs, int device, void *stream);
 

@@ -200,6 +200,10 @@ extern "C" int uavsim_policy_sample(const float *obs, int64_t rows, const UavSim
   int rc = policy_check_weights(w, "uavsim_policy_sample");
   if (rc) return rc;
   if (rows == 0) return 0;
+  if ((reinterpret_cast<uintptr_t>(obs) & 15) != 0) {  // the kernel reads each row with three float4 loads
+    SET_ERR("uavsim_policy_sample: obs must be 16-byte aligned");
+    return UAVSIM_ERR_ARG;
+  }
   CUDA_TRY(cudaSetDevice(device));
   const PolicyDev W = policy_dev(w);
   PolicyLaunch L;

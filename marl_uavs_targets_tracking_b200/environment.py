@@ -330,7 +330,7 @@ class BatchedEnvironment:
                 raise ValueError("run_policy: %s must be a contiguous %s tensor of shape %s on %s (got %s %s on %s)"
                                  % (name, dtype, shape, self.device, t.dtype, tuple(t.shape), t.device))
             setattr(traj, name, t.data_ptr())
-        w, params = policy_weights(policy, self.state_dim)  # (params: kept alive over the call)
+        w, params = policy_weights(policy, self.state_dim, self.device)  # (params: kept alive over the call)
         self._sync_weights(config)
         mode, coop = self._mode(config, pmi)
         with self._on_device():

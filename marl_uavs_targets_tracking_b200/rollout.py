@@ -41,14 +41,16 @@ class ValueNet(nn.Module):
         return self.fc2(F.relu(self.fc1(x))).squeeze(1)
 
 
-def policy_weights(policy, state_dim):
+def policy_weights(policy, state_dim, device=None):
     """The UavSimPolicyWeights of a PolicyNet (or a DDP wrapper around one) and the tensors it points into, which the
-    caller keeps alive while the struct is in use."""
+    caller keeps alive while the struct is in use.  The kernel reads contiguous float32 on `device` (default: where the
+    parameters are): parameters of another dtype, layout or device are converted into fresh tensors (a .double() or
+    .half() net would otherwise be read as float32 bit patterns); parameters that already are so are used in place."""
     net = policy.module if hasattr(policy, "module") else policy
     w = _cabi.UavSimPolicyWeights()
     w.state_dim, w.hidden, w.n_actions = state_dim, net.fc1.out_features, net.fc2.out_features
     params = [net.fc1.weight, net.fc1.bias, net.fc2.weight, net.fc2.bias]
-    params = [p.detach() if p.is_contiguous() else p.detach().contiguous() for p in params]
+    params = [p.detach().to(device=device, dtype=torch.float32).contiguous() for p in params]
     w.w1, w.b1, w.w2, w.b2 = (p.data_ptr() for p in params)
     return w, params
 
@@ -59,10 +61,12 @@ def fused_policy_sample(policy, states, seed, counter, want_probs=False, out=Non
     (or a DDP wrapper around one) on the device of `states` [B,12] float32; `out` = a contiguous int32 [B] tensor to write
     the actions into (e.g. the environment's bound action buffer).  Returns (actions int32 [B], probs or None)."""
     x = states if (states.dtype == torch.float32 and states.is_contiguous()) else states.float().contiguous()
+    if x.data_ptr() % 16:  # the kernel reads rows with 16-byte loads: a view off a 16-byte boundary is copied
+        x = x.clone()
     dev = x.device
     if dev.type != "cuda":
         raise _cabi.UavSimError("fused_policy_sample needs CUDA tensors (no CPU fallback)")
-    w, params = policy_weights(policy, x.shape[1])
+    w, params = policy_weights(policy, x.shape[1], dev)
     B, A = x.shape[0], w.n_actions
     if out is not None:
         assert out.dtype == torch.int32 and out.is_contiguous() and out.numel() == B and out.device == dev
@@ -94,8 +98,10 @@ class BatchedActorCritic:
         self.critic_optimizer = torch.optim.Adam(self.critic.parameters(), lr=critic_lr)
         self.gamma, self.device = gamma, device
         # rollout policy step: the fused kernel draws from Philox (seed; row, call number); fused=False is the stock
-        # torch forward + multinomial
-        self.fused = bool(fused) and torch.device(device).type == "cuda" and state_dim == 12 and action_dim <= 16
+        # torch forward + multinomial, which also serves the sizes the kernel does not (csrc/policy.cuh: 12 inputs,
+        # 1..512 hidden units, 2..16 actions)
+        self.fused = (bool(fused) and torch.device(device).type == "cuda" and state_dim == 12 and 1 <= hidden_dim <= 512
+                      and 2 <= action_dim <= 16)
         # Every rank rolls out its own environments: the draws of rank r must differ from rank 0's (the Philox counter
         # is the LOCAL row), so the rank is folded into the seed.
         import torch.distributed as dist

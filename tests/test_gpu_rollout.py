@@ -61,48 +61,6 @@ def test_reference_training_loop_on_the_device():
     env.close()
 
 
-@pytest.mark.parametrize("hidden,na,rows", [(128, 12, 100_003), (64, 12, 7), (128, 5, 4097), (256, 16, 1000)])
-def test_fused_policy_kernel_matches_torch_forward_and_draws_from_it(hidden, na, rows):
-    """uavsim_policy_sample: probabilities equal torch's softmax(fc2(relu(fc1(x)))) to fp32 rounding, the action of every
-    row is the inverse-CDF draw for its Philox uniform, and the empirical action frequencies follow the probabilities."""
-    import numpy as np
-    from philox_ref import philox4x32_10, u53
-    from marl_uavs_targets_tracking_b200.rollout import PolicyNet, fused_policy_sample
-    dev = torch.device("cuda:0")
-    torch.manual_seed(hidden + na)
-    net = PolicyNet(12, hidden, na).to(dev)
-    x = torch.randn(rows, 12, device=dev)
-    act, probs = fused_policy_sample(net, x, seed=99, counter=5, want_probs=True)
-    with torch.no_grad():
-        ref = net(x)
-    assert act.dtype == torch.int32 and act.shape == (rows,) and probs.shape == (rows, na)
-    assert float((probs - ref).abs().max()) <= 2e-6
-    assert 0 <= int(act.min()) and int(act.max()) < na
-    # the draw: u = philox_u53(seed; row, counter); action = #prefix sums of the kernel's own probabilities <= u
-    r = np.arange(rows)
-    x4 = philox4x32_10(r, 0, 5, 0, 99)
-    u = u53(x4[0], x4[1]).astype(np.float32)
-    cdf = np.cumsum(probs.double().cpu().numpy(), axis=1)
-    expect = np.minimum((cdf[:, :-1] <= u[:, None].astype(np.float64)).sum(1), na - 1)
-    got = act.cpu().numpy()
-    # float32 prefix sums in the kernel vs float64 here: a uniform within ~1e-7 of a boundary may land next door
-    assert (got != expect).mean() <= 1e-4 and np.abs(got - expect).max() <= 1
-    # a different counter gives different draws; the same one is reproducible
-    act2, _ = fused_policy_sample(net, x, seed=99, counter=6)
-    act3, _ = fused_policy_sample(net, x, seed=99, counter=5)
-    assert torch.equal(act, act3)
-    if rows > 1000:
-        assert float((act != act2).float().mean()) > 0.5
-        # frequencies: same input row repeated -> chi-square against its probability vector
-        xr = x[:1].repeat(200_000, 1).contiguous()
-        a, p = fused_policy_sample(net, xr, seed=1, counter=1, want_probs=True)
-        cnt = torch.bincount(a.long(), minlength=na).double().cpu().numpy()
-        e = p[0].double().cpu().numpy() * 200_000
-        keep = e > 5
-        chi2 = (((cnt - e) ** 2 / np.maximum(e, 1e-30))[keep]).sum()
-        assert chi2 < 60, (chi2, cnt, e)
-
-
 def test_rollout_paths_agree():
     """keep_transitions on/off and the stock torch policy step drive the same environment dynamics: with the fused
     policy (Philox draws keyed by call number) the two modes visit identical states."""
