@@ -4,8 +4,8 @@ the generic kernel.
 
 The fast kernel classifies every pair in fp32 with a two-sided guard and sends a UAV to the fp64 path only when a
 pair falls inside the guard band; these tests pin (i) both template instances (plain, and with masks / per-target
-counts) to the oracle, (ii) the two kernels to each other on every integer output, and (iii) the fp64 path itself by
-placing pairs EXACTLY on the thresholds (d == dp, d == dc, d == 2 dp after the move), where `<=` and `<` differ.
+counts) to the oracle and (ii) the two kernels to each other on every integer output.  Pairs placed exactly on the
+thresholds, for these and the other step kernels, are in test_gpu_pair_thresholds.py.
 """
 import numpy as np
 import pytest
@@ -96,63 +96,6 @@ def test_fast_and_generic_kernels_agree(fast_path):
         assert abs(a[k] - b[k]) <= 1e-6 * max(1.0, abs(a[k]))
     g.close()
     f.close()
-
-
-@pytest.mark.parametrize("path", PATHS)
-def test_pairs_exactly_on_the_thresholds(oracle, path):
-    """Entities placed so that AFTER the move d == dp (observe / track: inside; coverage: outside), d == dc for a
-    partner that moved first and for one observed at its old position, d == 2 dp and d == dp between UAVs -- and the
-    same geometry one ulp inside / outside.  Headings 0 / pi/2 keep the moves exact (cos 0 = 1, sin 0 = 0), so the
-    distances are exactly on the thresholds and only the fp64 path can decide them."""
-    from marl_uavs_targets_tracking_b200 import default_config
-    n = m = 64
-    cfg = default_config("MAAC-G", n, m)
-    E = 7
-    env = _env(n, m, cfg, E, seed=1, record_masks=True, track_counts=True)
-    env.set_step_path(path)
-    env.reset(cfg)
-    st = {k: v.cpu().numpy().copy() for k, v in env.get_state().items()}
-    # park everything far apart first (a sparse lattice outside each other's ranges where possible)
-    for e in range(E):
-        st["uh"][e, :] = 0.0
-        st["th"][e, :] = 0.0
-        st["ux"][e, :] = 100.0 + 29.0 * np.arange(n)
-        st["uy"][e, :] = 1900.0
-        st["tx"][e, :] = 50.0 + 30.0 * np.arange(m)
-        st["ty"][e, :] = 50.0
-    up = np.nextafter
-    for e, eps in enumerate((0.0, 1.0, -1.0, 0.0, 1.0, -1.0, 0.0)):
-        def nudge(v, _eps=eps):  # one ulp in or out
-            return v if _eps == 0 else float(up(v, v + _eps))
-        # UAV 10 ends at (1000, 1000); target 5 ends at (1200 (+-ulp), 1000): d == dp
-        st["ux"][e, 10], st["uy"][e, 10] = 980.0, 1000.0
-        st["tx"][e, 5], st["ty"][e, 5] = nudge(1195.0), 1000.0
-        # UAV 3 (moves before 10) ends at (1000, 1500 (+-ulp)): d == dc, new-new
-        st["ux"][e, 3], st["uy"][e, 3] = 980.0, nudge(1500.0)
-        # UAV 20 (moves after 10) observed at its OLD position (1000, 500 (+-ulp)): d == dc, new-old
-        st["ux"][e, 20], st["uy"][e, 20] = 1000.0, nudge(500.0)
-        # UAV 30 ends at (1400 (+-ulp), 1000): d == 2 dp ; UAV 40 ends at (800 (+-ulp), 1000): d == dp
-        st["ux"][e, 30], st["uy"][e, 30] = nudge(1380.0), 1000.0
-        st["ux"][e, 40], st["uy"][e, 40] = nudge(780.0), 1000.0
-    env.set_state(cfg, *(st[k] for k in ("ux", "uy", "uh", "ua", "tx", "ty", "th")))
-    P = oracle_params_from_config(cfg, n, m)
-    a = np.full((E, n), 5, np.int32)
-    obs, rew4, cov = env.step_device(cfg, None, torch.as_tensor(a, device="cuda:0"))
-    host = {k: np.ascontiguousarray(v) for k, v in st.items()}
-    seen = set()
-    for e in range(E):
-        one = {k: host[k][e].copy() for k in host}
-        ref = oracle.step(P, 1, float(cfg["cooperative"]), None, one, a[e], masks=True)
-        for k in MASKS:
-            assert np.array_equal(env.masks[k][e].cpu().numpy(), ref[k]), (e, k)
-        assert int(cov[e]) == ref["covered"]
-        assert np.array_equal(env.tracker_counts[e].cpu().numpy(), ref["tracker_cnt"])
-        assert max_scaled_err(obs[e].double().cpu().numpy(), ref["obs"]) <= TOL_TIGHT
-        seen.add((int(ref["obs_mask"][10, 5]), int(ref["cover_mask"][10, 5]), int(ref["comm_mask"][10, 3]),
-                  int(ref["comm_mask"][10, 20]), int(ref["dup_mask"][10, 30]), int(ref["nbr_mask"][10, 40])))
-    # the three variants really fall on different sides: on the threshold (<= true, < false), inside, outside
-    assert (1, 0, 1, 1, 1, 1) in seen and len(seen) >= 2, seen
-    env.close()
 
 
 @pytest.mark.parametrize("path", PATHS)
