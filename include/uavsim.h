@@ -245,6 +245,12 @@ typedef struct {
 int uavsim_policy_sample(const float *obs, int64_t rows, const UavSimPolicyWeights *w, uint64_t seed, uint64_t counter,
                          int32_t *actions, float *probs, int device, void *stream);
 
+/* Greedy twin of uavsim_policy_sample, the deterministic action rule of evaluation: actions[r] = the smallest index among
+ * the maximal probabilities of row r as the kernel computes them, i.e. torch.argmax of the probs output (NULL allowed).
+ * Same argument checks; no random draw. */
+int uavsim_policy_greedy(const float *obs, int64_t rows, const UavSimPolicyWeights *w, int32_t *actions, float *probs,
+                         int device, void *stream);
+
 /* Device trajectory buffers of uavsim_run_policy (T = nsteps); any field may be NULL: that output then goes to the
  * bound buffer, overwritten step by step.  obs must be 16-byte aligned, like the bound observation buffer. */
 typedef struct UavSimTrajectory {
@@ -272,6 +278,28 @@ typedef struct UavSimTrajectory {
  * launches count in uavsim_launch_count. */
 int uavsim_run_policy(uavsim_t *h, int mode, double cooperative, const UavSimPolicyWeights *w, uint64_t seed,
                       uint64_t first_counter, int64_t nsteps, const UavSimTrajectory *traj, void *stream);
+
+/* Evaluation of a policy over many episodes in one call (the reference's `--phase evaluate`, src/train.py evaluate, for
+ * all environments at once), in place on the bound buffers: for k = 0 .. n_episodes-1
+ *     uavsim_reset(h, reset_seeds[k], stream);
+ *     nsteps x (policy launch -> bound actions; uavsim_step; per-environment accumulation)
+ * greedy = 0: step t of episode k draws as uavsim_policy_sample with counter first_counter + k*nsteps + t, i.e. each
+ * episode is uavsim_run_policy(h, mode, cooperative, w, seed, first_counter + k*nsteps, nsteps, NULL, stream);
+ * greedy = 1: uavsim_policy_greedy (seed and first_counter unused).  reset_seeds: HOST array [n_episodes].
+ * env_stats: DEVICE float64 [n_episodes, E, 6], 8-byte aligned: per environment the sums over UAVs and steps of the four
+ * reward planes (rewards, target_tracking, boundary, duplicate; as the statistics hold them: counts of 2^-22 of the fp32
+ * values), the covered-target sum and the covered-target maximum over steps.  These are the integers the episode
+ * statistics add up, so for every episode the sum of its rows over environments equals uavsim_episode_stats out[0..4]
+ * and their maximum out[5], bit for bit, whichever step kernel ran.
+ * The result is bit-identical to the loop above in the bound obs / actions / rew4 / covered, done, the state, the step
+ * counter and uavsim_episode_stats (which hold the last episode).  uavsim_launch_count counts the loop's launches plus
+ * nsteps + 1 per episode (the accumulation and the row output).  Every argument is checked before anything is queued
+ * (negative counts, NULL reset_seeds / env_stats when n_episodes > 0, a misaligned env_stats, greedy not 0 / 1, the
+ * weights, n_actions != na, the PMI path): on an error nothing is enqueued and the step counter does not move.
+ * n_episodes = 0 queues nothing.  The handle keeps an [E,6] int64 accumulator, allocated on the first call. */
+int uavsim_evaluate_policy(uavsim_t *h, int mode, double cooperative, const UavSimPolicyWeights *w, int greedy,
+                           uint64_t seed, uint64_t first_counter, const uint64_t *reset_seeds, int64_t n_episodes,
+                           int64_t nsteps, double *env_stats, void *stream);
 
 #ifdef __cplusplus
 }

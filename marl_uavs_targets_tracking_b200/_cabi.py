@@ -76,6 +76,11 @@ SYMBOLS = {
                                        C.c_void_p, C.c_void_p, C.c_int, C.c_void_p]),
     "uavsim_run_policy": (C.c_int, [_H, C.c_int, C.c_double, C.POINTER(UavSimPolicyWeights), C.c_uint64, C.c_uint64,
                                     C.c_int64, C.POINTER(UavSimTrajectory), C.c_void_p]),
+    "uavsim_policy_greedy": (C.c_int, [C.c_void_p, C.c_int64, C.POINTER(UavSimPolicyWeights), C.c_void_p, C.c_void_p,
+                                       C.c_int, C.c_void_p]),
+    "uavsim_evaluate_policy": (C.c_int, [_H, C.c_int, C.c_double, C.POINTER(UavSimPolicyWeights), C.c_int, C.c_uint64,
+                                         C.c_uint64, C.POINTER(C.c_uint64), C.c_int64, C.c_int64, C.c_void_p,
+                                         C.c_void_p]),
     # prioritized replay (src/train.py:73-139)
     "uavsim_replay_create": (C.c_int, [C.c_int64, C.c_int, C.c_double, C.c_int, C.POINTER(_H)]),
     "uavsim_replay_destroy": (C.c_int, [_H]),

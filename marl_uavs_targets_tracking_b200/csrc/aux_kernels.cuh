@@ -88,3 +88,41 @@ __global__ void uavsim_stats_reduce_kernel(const long long *__restrict__ stats, 
   __syncthreads();
   if (threadIdx.x < STAT_W) out[threadIdx.x] = (double)tot[threadIdx.x] * (threadIdx.x <= ST_DUP ? 1.0 / 4194304.0 : 1.0);
 }
+
+// Per-environment statistics of an evaluation (uavsim_evaluate_policy), accumulated after every step into acc [E][6]
+// int64: the four reward planes as sums over UAVs of sf_fx -- the integers the step and PMI kernels commit through
+// stats_commit -- then covered targets summed and their maximum over steps.  Summed over environments the rows are
+// therefore exactly the episode statistics, whichever kernel served the step.  One warp per environment with the lanes
+// over UAVs (a 64-UAV swarm is two values per lane), grid-stride over environments; lane k < 6 writes field k.
+#define ENV_ACC_W 6
+__global__ void uavsim_env_stats_kernel(const KParams P, const float *__restrict__ rew4, const int32_t *__restrict__ covered,
+                                        long long *__restrict__ acc) {
+  const int lane = threadIdx.x & 31;
+  const int64_t plane = P.E * P.n;
+  const int64_t wstride = (int64_t)gridDim.x * (blockDim.x >> 5);
+  for (int64_t e = ((int64_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5; e < P.E; e += wstride) {
+    long long v[4] = {0, 0, 0, 0};
+    for (int i = lane; i < P.n; i += 32)
+#pragma unroll
+      for (int q = 0; q < 4; q++) v[q] += sf_fx(rew4[q * plane + e * P.n + i]);
+#pragma unroll
+    for (int q = 0; q < 4; q++)
+#pragma unroll
+      for (int o = 16; o > 0; o >>= 1) v[q] += __shfl_xor_sync(0xffffffffu, v[q], o);
+    if (lane < ENV_ACC_W) {
+      long long *a = acc + e * ENV_ACC_W + lane;
+      if (lane < 4) *a += lane == 0 ? v[0] : lane == 1 ? v[1] : lane == 2 ? v[2] : v[3];
+      else if (lane == 4) *a += covered[e];
+      else *a = max(*a, (long long)covered[e]);
+    }
+  }
+}
+
+// End of an evaluated episode: its row of the output as float64 (counts x 2^-22, exact) and the accumulators cleared.
+__global__ void uavsim_env_stats_finish_kernel(long long *__restrict__ acc, int64_t count, double *__restrict__ out) {
+  const int64_t stride = (int64_t)gridDim.x * blockDim.x;
+  for (int64_t k = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; k < count; k += stride) {
+    out[k] = (double)acc[k] * (k % ENV_ACC_W < 4 ? 1.0 / 4194304.0 : 1.0);
+    acc[k] = 0;
+  }
+}

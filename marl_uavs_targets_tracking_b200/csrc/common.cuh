@@ -104,6 +104,7 @@ struct uavsim {
   double *d_stats8;   // [8] reduced
   double *h_stats8;   // pinned
   int stat_slots;
+  long long *d_env_acc; // [E][6] per-environment statistics of uavsim_evaluate_policy (allocated on first use)
   int epb, grid_max, nt;   // environments per CTA, resident CTAs, threads per CTA of the step kernel
   StepKernelFn step_fn[2];  // [MASKS]
   size_t smem_step;

@@ -45,10 +45,12 @@ __device__ __forceinline__ float pol_hi(uint64_t v) { return __uint_as_float((ui
 // PDL: the form uavsim_run_policy launches with programmatic dependent launch.  The weights are constant for the whole
 // call, so they are staged before griddepcontrol.wait and that overlaps the previous step kernel's tail; nothing else
 // touches global memory before the wait.  Launched without the attribute, the wait passes straight through.
-template <int AP, bool PDL = false>
-__global__ void __launch_bounds__(POLICY_NT)
-uavsim_policy_kernel(const float *__restrict__ obs, int64_t rows, const PolicyDev W, uint64_t seed, uint64_t counter,
-                     int32_t *__restrict__ actions, float *__restrict__ probs) {
+// GREEDY: the deterministic action rule of evaluation.  The same logits and softmax; the action is the smallest index
+// among the maximal probabilities as this kernel computes them (lg[a] * (1 / sum), the values the probs output holds), so
+// it equals torch.argmax of that output.  No Philox draw: seed and counter are ignored.
+template <int AP, bool PDL, bool GREEDY>
+__device__ __forceinline__ void policy_rows(const float *__restrict__ obs, int64_t rows, const PolicyDev W, uint64_t seed,
+                                            uint64_t counter, int32_t *__restrict__ actions, float *__restrict__ probs) {
   extern __shared__ __align__(16) float s_w[];
   const int H = W.H, A = W.A, HP = (H + 1) / 2;  // unit pairs (an odd H gets a zero unit: relu(0) * 0 adds nothing)
   for (int k = threadIdx.x; k < HP * 64; k += POLICY_NT) {
@@ -119,14 +121,24 @@ uavsim_policy_kernel(const float *__restrict__ obs, int64_t rows, const PolicyDe
       float sum = 0.f;
 #pragma unroll
       for (int a = 0; a < AP; a++) { lg[a] = expf(lg[a] - mx); sum += lg[a]; }
-      const Philox4 rn = philox4x32_10((uint32_t)r, (uint32_t)(r >> 32), (uint32_t)counter, (uint32_t)(counter >> 32), seed);
-      // (the 53-bit uniform can round UP to 1.0f: clamped below 1, or a zero-probability last action could be drawn)
-      const float u = fminf((float)philox_u53(rn.v[0], rn.v[1]), 0x1.fffffep-1f) * sum;
-      // inverse CDF: the action is the number of prefix sums that do not exceed u, capped at the last action
-      float run = 0.f;
       int act = 0;
+      if constexpr (GREEDY) {
+        const float inv = 1.0f / sum;
+        float best = lg[0] * inv;
 #pragma unroll
-      for (int a = 0; a < AP - 1; a++) { run += lg[a]; act += (run <= u && a < A - 1) ? 1 : 0; }
+        for (int a = 1; a < AP; a++) {
+          const float p = lg[a] * inv;
+          if (a < A && p > best) { best = p; act = a; }  // strictly greater: a tie keeps the first index
+        }
+      } else {
+        const Philox4 rn = philox4x32_10((uint32_t)r, (uint32_t)(r >> 32), (uint32_t)counter, (uint32_t)(counter >> 32), seed);
+        // (the 53-bit uniform can round UP to 1.0f: clamped below 1, or a zero-probability last action could be drawn)
+        const float u = fminf((float)philox_u53(rn.v[0], rn.v[1]), 0x1.fffffep-1f) * sum;
+        // inverse CDF: the action is the number of prefix sums that do not exceed u, capped at the last action
+        float run = 0.f;
+#pragma unroll
+        for (int a = 0; a < AP - 1; a++) { run += lg[a]; act += (run <= u && a < A - 1) ? 1 : 0; }
+      }
       actions[r] = act;
       if (probs) {
         const float inv = 1.0f / sum;
@@ -135,6 +147,21 @@ uavsim_policy_kernel(const float *__restrict__ obs, int64_t rows, const PolicyDe
       }
     }
   }
+}
+
+template <int AP, bool PDL = false>
+__global__ void __launch_bounds__(POLICY_NT)
+uavsim_policy_kernel(const float *__restrict__ obs, int64_t rows, const PolicyDev W, uint64_t seed, uint64_t counter,
+                     int32_t *__restrict__ actions, float *__restrict__ probs) {
+  policy_rows<AP, PDL, false>(obs, rows, W, seed, counter, actions, probs);
+}
+
+// The greedy form: a kernel of its own name, so that traces and profiles tell the two action rules apart.
+template <int AP, bool PDL = false>
+__global__ void __launch_bounds__(POLICY_NT)
+uavsim_policy_greedy_kernel(const float *__restrict__ obs, int64_t rows, const PolicyDev W, uint64_t seed,
+                            uint64_t counter, int32_t *__restrict__ actions, float *__restrict__ probs) {
+  policy_rows<AP, PDL, true>(obs, rows, W, seed, counter, actions, probs);
 }
 
 // ------------------------------------------------------------------------------------------------
@@ -167,12 +194,21 @@ static PolicyDev policy_dev(const UavSimPolicyWeights *w) {
 }
 
 // (weights already checked by policy_check_weights; needs the current device set)
-static int policy_plan(int64_t rows, const PolicyDev &W, bool pdl, int device, PolicyLaunch *L) {
-  switch ((W.A + 3) / 4) {
-    case 1: L->fn = pdl ? uavsim_policy_kernel<4, true> : uavsim_policy_kernel<4>; break;
-    case 2: L->fn = pdl ? uavsim_policy_kernel<8, true> : uavsim_policy_kernel<8>; break;
-    case 3: L->fn = pdl ? uavsim_policy_kernel<12, true> : uavsim_policy_kernel<12>; break;
-    default: L->fn = pdl ? uavsim_policy_kernel<16, true> : uavsim_policy_kernel<16>; break;
+static int policy_plan(int64_t rows, const PolicyDev &W, bool pdl, bool greedy, int device, PolicyLaunch *L) {
+  if (greedy) {
+    switch ((W.A + 3) / 4) {
+      case 1: L->fn = pdl ? uavsim_policy_greedy_kernel<4, true> : uavsim_policy_greedy_kernel<4>; break;
+      case 2: L->fn = pdl ? uavsim_policy_greedy_kernel<8, true> : uavsim_policy_greedy_kernel<8>; break;
+      case 3: L->fn = pdl ? uavsim_policy_greedy_kernel<12, true> : uavsim_policy_greedy_kernel<12>; break;
+      default: L->fn = pdl ? uavsim_policy_greedy_kernel<16, true> : uavsim_policy_greedy_kernel<16>; break;
+    }
+  } else {
+    switch ((W.A + 3) / 4) {
+      case 1: L->fn = pdl ? uavsim_policy_kernel<4, true> : uavsim_policy_kernel<4>; break;
+      case 2: L->fn = pdl ? uavsim_policy_kernel<8, true> : uavsim_policy_kernel<8>; break;
+      case 3: L->fn = pdl ? uavsim_policy_kernel<12, true> : uavsim_policy_kernel<12>; break;
+      default: L->fn = pdl ? uavsim_policy_kernel<16, true> : uavsim_policy_kernel<16>; break;
+    }
   }
   L->smem = (size_t)((W.H + 1) / 2) * 64 * sizeof(float);
   int rc = raise_dynamic_smem((const void *)L->fn, device, L->smem);
@@ -191,25 +227,37 @@ static int policy_plan(int64_t rows, const PolicyDev &W, bool pdl, int device, P
   return 0;
 }
 
-extern "C" int uavsim_policy_sample(const float *obs, int64_t rows, const UavSimPolicyWeights *w, uint64_t seed,
-                                    uint64_t counter, int32_t *actions, float *probs, int device, void *stream) {
+// uavsim_policy_sample / uavsim_policy_greedy: every argument is checked before the device is touched
+static int policy_launch_rows(const float *obs, int64_t rows, const UavSimPolicyWeights *w, bool greedy, uint64_t seed,
+                              uint64_t counter, int32_t *actions, float *probs, int device, void *stream,
+                              const char *who) {
   if (!w || rows < 0 || (rows > 0 && (!obs || !actions))) {
-    SET_ERR("uavsim_policy_sample: NULL argument");
+    SET_ERR("%s: NULL argument", who);
     return UAVSIM_ERR_ARG;
   }
-  int rc = policy_check_weights(w, "uavsim_policy_sample");
+  int rc = policy_check_weights(w, who);
   if (rc) return rc;
   if (rows == 0) return 0;
   if ((reinterpret_cast<uintptr_t>(obs) & 15) != 0) {  // the kernel reads each row with three float4 loads
-    SET_ERR("uavsim_policy_sample: obs must be 16-byte aligned");
+    SET_ERR("%s: obs must be 16-byte aligned", who);
     return UAVSIM_ERR_ARG;
   }
   CUDA_TRY(cudaSetDevice(device));
   const PolicyDev W = policy_dev(w);
   PolicyLaunch L;
-  rc = policy_plan(rows, W, false, device, &L);
+  rc = policy_plan(rows, W, false, greedy, device, &L);
   if (rc) return rc;
   L.fn<<<L.blocks, POLICY_NT, L.smem, (cudaStream_t)stream>>>(obs, rows, W, seed, counter, actions, probs);
   CUDA_TRY(cudaGetLastError());
   return 0;
+}
+
+extern "C" int uavsim_policy_sample(const float *obs, int64_t rows, const UavSimPolicyWeights *w, uint64_t seed,
+                                    uint64_t counter, int32_t *actions, float *probs, int device, void *stream) {
+  return policy_launch_rows(obs, rows, w, false, seed, counter, actions, probs, device, stream, "uavsim_policy_sample");
+}
+
+extern "C" int uavsim_policy_greedy(const float *obs, int64_t rows, const UavSimPolicyWeights *w, int32_t *actions,
+                                    float *probs, int device, void *stream) {
+  return policy_launch_rows(obs, rows, w, true, 0, 0, actions, probs, device, stream, "uavsim_policy_greedy");
 }

@@ -335,6 +335,7 @@ extern "C" int uavsim_destroy(uavsim_t *h) {
   if (!h) return 0;
   cudaSetDevice(h->device);
   cudaFree(h->d_dth); cudaFree(h->d_act); cudaFree(h->d_sctab); cudaFree(h->d_fast_ctr); cudaFree(h->d_stats); cudaFree(h->d_stats8); cudaFreeHost(h->h_stats8);
+  cudaFree(h->d_env_acc);
   cudaFree(h->d_pmi_blob); cudaFree(h->d_tc_tiles);
   if (h->s_in) cudaStreamDestroy(h->s_in);
   if (h->s_comp) cudaStreamDestroy(h->s_comp);
@@ -829,20 +830,47 @@ extern "C" int uavsim_run_random_policy(uavsim_t *h, int mode, double coop, uint
   return 0;
 }
 
+// The weights of a policy loop: the fused kernel's rules, and one logit per action of the environment.
+static int policy_loop_weights(const uavsim_t *h, const UavSimPolicyWeights *w, const char *who) {
+  const int rc = policy_check_weights(w, who);
+  if (rc) return rc;
+  if (w->n_actions != h->kp.na) { SET_ERR("%s: the policy has %d actions, the environment na = %d", who, w->n_actions, h->kp.na); return UAVSIM_ERR_ARG; }
+  return 0;
+}
+
+// One step of a learned-policy loop (uavsim_run_policy, uavsim_evaluate_policy): the policy launch reading `obs` and
+// writing the bound action buffer, then the step kernel chosen exactly as uavsim_step chooses it -- not with the wider
+// small-kernel range of the random-policy loop, whose draw is fused into that kernel -- so every output is bit-identical
+// to the per-step calls.  The first policy launch of a loop follows the caller's own work (which may have just written
+// the weights): `pdl` false, a plain launch.  Later ones follow the loop's own kernels and may start early.
+static int policy_then_step(uavsim_t *h, int mode, double coop, const PolicyLaunch &L, const PolicyDev &W,
+                            const float *obs, uint64_t seed, uint64_t counter, bool pdl, cudaStream_t st, const char *who) {
+  cudaLaunchConfig_t cfg = {};
+  cfg.gridDim = dim3((unsigned)L.blocks); cfg.blockDim = dim3(POLICY_NT); cfg.dynamicSmemBytes = L.smem; cfg.stream = st;
+  cudaLaunchAttribute at[1];
+  at[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
+  at[0].val.programmaticStreamSerializationAllowed = pdl ? 1 : 0;
+  cfg.attrs = at; cfg.numAttrs = 1;
+  float *no_probs = nullptr;
+  cudaError_t e = cudaLaunchKernelEx(&cfg, L.fn, obs, h->E * h->kp.n, W, seed, counter, h->buf.actions, no_probs);
+  if (e != cudaSuccess) { SET_ERR("%s: policy launch failed: %s", who, cudaGetErrorString(e)); return (int)e; }
+  h->launches++;
+  h->t++;
+  const int done = (h->hp.num_steps > 0 && h->t >= h->hp.num_steps) ? 1 : 0;
+  return launch_step_range(h, mode, coop, 0, h->E, done, st, true);
+}
+
 // Learned-policy rollout below the FFI: nsteps x (policy launch, step) queued back to back.  The handle's bound
 // obs / actions / rew4 / covered pointers are pointed at the trajectory slots of each step (the kernels take the buffer
-// struct by value, so this costs nothing) and restored before returning.  The step kernel is chosen exactly as
-// uavsim_step chooses it -- not with the wider small-kernel range of the random-policy loop, whose draw is fused into
-// that kernel -- so every output is bit-identical to the per-step calls.
+// struct by value, so this costs nothing) and restored before returning.
 extern "C" int uavsim_run_policy(uavsim_t *h, int mode, double coop, const UavSimPolicyWeights *w, uint64_t seed,
                                  uint64_t first_counter, int64_t nsteps, const UavSimTrajectory *traj, void *stream) {
   const char *who = "uavsim_run_policy";
   int rc = check_step_args(h, mode, coop, who);
   if (rc) return rc;
   if (nsteps < 0) { SET_ERR("%s: nsteps < 0", who); return UAVSIM_ERR_ARG; }
-  rc = policy_check_weights(w, who);
+  rc = policy_loop_weights(h, w, who);
   if (rc) return rc;
-  if (w->n_actions != h->kp.na) { SET_ERR("%s: the policy has %d actions, the environment na = %d", who, w->n_actions, h->kp.na); return UAVSIM_ERR_ARG; }
   const UavSimTrajectory tr = traj ? *traj : UavSimTrajectory{nullptr, nullptr, nullptr, nullptr};
   if ((reinterpret_cast<uintptr_t>(tr.obs) & 15) != 0) { SET_ERR("%s: trajectory obs must be 16-byte aligned", who); return UAVSIM_ERR_ARG; }
   const UavSimBuffers home = h->buf;
@@ -872,7 +900,7 @@ extern "C" int uavsim_run_policy(uavsim_t *h, int mode, double coop, const UavSi
   CUDA_TRY(cudaSetDevice(h->device));
   const PolicyDev W = policy_dev(w);
   PolicyLaunch L;
-  rc = policy_plan(en, W, true, h->device, &L);
+  rc = policy_plan(en, W, true, false, h->device, &L);
   if (rc) return rc;
 
   cudaStream_t st = (cudaStream_t)stream;
@@ -880,21 +908,7 @@ extern "C" int uavsim_run_policy(uavsim_t *h, int mode, double coop, const UavSi
   for (int64_t k = 0; k < nsteps && rc == 0; k++) {
     const float *obs_k = tr.obs ? tr.obs + k * en * 12 : home.obs;
     bind_slot(k);
-    // The first policy launch follows the caller's own work (which may have just written the weights): a plain launch.
-    // Later ones follow this loop's step or PMI kernel and may start early.
-    cudaLaunchConfig_t cfg = {};
-    cfg.gridDim = dim3((unsigned)L.blocks); cfg.blockDim = dim3(POLICY_NT); cfg.dynamicSmemBytes = L.smem; cfg.stream = st;
-    cudaLaunchAttribute at[1];
-    at[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-    at[0].val.programmaticStreamSerializationAllowed = k > 0 ? 1 : 0;
-    cfg.attrs = at; cfg.numAttrs = 1;
-    float *no_probs = nullptr;
-    cudaError_t e = cudaLaunchKernelEx(&cfg, L.fn, obs_k, en, W, seed, first_counter + (uint64_t)k, h->buf.actions, no_probs);
-    if (e != cudaSuccess) { SET_ERR("%s: policy launch failed: %s", who, cudaGetErrorString(e)); rc = (int)e; break; }
-    h->launches++;
-    h->t++;
-    const int done = (h->hp.num_steps > 0 && h->t >= h->hp.num_steps) ? 1 : 0;
-    rc = launch_step_range(h, mode, coop, 0, E, done, st, true);
+    rc = policy_then_step(h, mode, coop, L, W, obs_k, seed, first_counter + (uint64_t)k, k > 0, st, who);
   }
   h->buf = home;
   if (rc || nsteps == 0) return rc;
@@ -903,6 +917,58 @@ extern "C" int uavsim_run_policy(uavsim_t *h, int mode, double coop, const UavSi
   if (tr.actions) CUDA_TRY(cudaMemcpyAsync(home.actions, tr.actions + (nsteps - 1) * en, sizeof(int32_t) * en, cudaMemcpyDeviceToDevice, st));
   if (tr.rew4) CUDA_TRY(cudaMemcpyAsync(home.rew4, tr.rew4 + (nsteps - 1) * 4 * en, sizeof(float) * 4 * en, cudaMemcpyDeviceToDevice, st));
   if (tr.covered) CUDA_TRY(cudaMemcpyAsync(home.covered, tr.covered + (nsteps - 1) * E, sizeof(int32_t) * E, cudaMemcpyDeviceToDevice, st));
+  return 0;
+}
+
+// Evaluation of a policy over n_episodes episodes in one call: per episode uavsim_reset, then the steps of
+// uavsim_run_policy (the same per-step body, in place on the bound buffers), each followed by the per-environment
+// accumulation, and one launch that writes the episode's rows and clears the accumulators.
+extern "C" int uavsim_evaluate_policy(uavsim_t *h, int mode, double coop, const UavSimPolicyWeights *w, int greedy,
+                                      uint64_t seed, uint64_t first_counter, const uint64_t *reset_seeds,
+                                      int64_t n_episodes, int64_t nsteps, double *env_stats, void *stream) {
+  const char *who = "uavsim_evaluate_policy";
+  int rc = check_step_args(h, mode, coop, who);
+  if (rc) return rc;
+  if (n_episodes < 0 || nsteps < 0) { SET_ERR("%s: n_episodes < 0 or nsteps < 0", who); return UAVSIM_ERR_ARG; }
+  if (greedy != 0 && greedy != 1) { SET_ERR("%s: greedy must be 0 or 1 (got %d)", who, greedy); return UAVSIM_ERR_ARG; }
+  if (n_episodes > 0 && (!reset_seeds || !env_stats)) { SET_ERR("%s: NULL reset_seeds or env_stats", who); return UAVSIM_ERR_ARG; }
+  if ((reinterpret_cast<uintptr_t>(env_stats) & 7) != 0) { SET_ERR("%s: env_stats must be 8-byte aligned", who); return UAVSIM_ERR_ARG; }
+  rc = policy_loop_weights(h, w, who);
+  if (rc) return rc;
+  if ((h->step_path == 2 || h->step_path == 3) && !fast_path_usable(h)) {
+    SET_ERR("%s: the selected step kernel needs 16-byte aligned bound buffers", who);
+    return UAVSIM_ERR_UNSUPPORTED;
+  }
+  if (mode == UAVSIM_MODE_PMI && coop != 0.0) {
+    rc = pmi_servable(h);
+    if (rc) return rc;
+  }
+  if (n_episodes == 0) return 0;
+  CUDA_TRY(cudaSetDevice(h->device));
+  const PolicyDev W = policy_dev(w);
+  PolicyLaunch L;
+  rc = policy_plan(h->E * h->kp.n, W, true, greedy == 1, h->device, &L);
+  if (rc) return rc;
+
+  cudaStream_t st = (cudaStream_t)stream;
+  const int64_t cells = h->E * ENV_ACC_W;
+  if (!h->d_env_acc) CUDA_TRY(cudaMalloc(&h->d_env_acc, sizeof(long long) * cells));
+  CUDA_TRY(cudaMemsetAsync(h->d_env_acc, 0, sizeof(long long) * cells, st));  // (whatever an interrupted call left)
+  const int acc_grid = elementwise_grid(h, h->E * 32), out_grid = elementwise_grid(h, cells);
+  for (int64_t k = 0; k < n_episodes; k++) {
+    rc = uavsim_reset(h, reset_seeds[k], stream);
+    if (rc) return rc;
+    for (int64_t t = 0; t < nsteps; t++) {
+      rc = policy_then_step(h, mode, coop, L, W, h->buf.obs, seed, first_counter + (uint64_t)(k * nsteps + t), t > 0, st, who);
+      if (rc) return rc;
+      uavsim_env_stats_kernel<<<acc_grid, 256, 0, st>>>(h->kp, h->buf.rew4, h->buf.covered, h->d_env_acc);
+      CUDA_TRY(cudaGetLastError());
+      h->launches++;
+    }
+    uavsim_env_stats_finish_kernel<<<out_grid, 256, 0, st>>>(h->d_env_acc, cells, env_stats + k * cells);
+    CUDA_TRY(cudaGetLastError());
+    h->launches++;
+  }
   return 0;
 }
 

@@ -179,12 +179,15 @@ class BatchedEnvironment:
         (seed, episode, global env id), so every episode and every environment differs but a run is
         reproducible for any number of GPUs."""
         self._ensure_handle(config)
-        s = self.seed if seed is None else int(seed)
-        ep_seed = (s * 0x9E3779B97F4A7C15 + self._episode * 0xD1B54A32D192ED03) & 0xFFFFFFFFFFFFFFFF
         with self._on_device():
-            _cabi.check(self._lib.uavsim_reset(self._h, C.c_uint64(ep_seed), self._stream()), "uavsim_reset")
+            _cabi.check(self._lib.uavsim_reset(self._h, C.c_uint64(self._episode_seed(seed, self._episode)),
+                                               self._stream()), "uavsim_reset")
         self._episode += 1
         self._clear_traces()
+
+    def _episode_seed(self, seed, episode):
+        s = self.seed if seed is None else int(seed)
+        return (s * 0x9E3779B97F4A7C15 + episode * 0xD1B54A32D192ED03) & 0xFFFFFFFFFFFFFFFF
 
     def set_state(self, config, ux, uy, uh, ua, tx, ty, th):
         """Replay path: load a recorded reset (e.g. the reference's `random`-module draws) for all envs."""
@@ -339,6 +342,40 @@ class BatchedEnvironment:
                         "uavsim_run_policy")
         self._host = None
         return self._obs, self._rew4, self._covered
+
+    def evaluate_policy(self, config, pmi, policy, n_episodes, nsteps, greedy=False, seed=None, first_counter=1,
+                        policy_seed=0):
+        """`n_episodes` evaluation episodes of `nsteps` steps in one library call (uavsim_evaluate_policy), equal bit for
+        bit to
+
+            for k in range(n_episodes):
+                env.reset(config, seed)
+                env.run_policy(config, pmi, policy, policy_seed, first_counter + k * nsteps, nsteps)
+
+        in the state, the bound buffers and episode_stats() (the last episode's); with greedy, every step takes the most
+        probable action (`fused_policy_greedy`) instead of a draw.  Episode k's reset seed is derived from `seed`
+        (default: the constructor's) exactly as reset() derives it, and the episode count advances by n_episodes.
+
+        Returns float64 [n_episodes, E, 6] on the device: per episode and environment the sums over UAVs and steps of the
+        four reward planes (rewards, target_tracking_reward, boundary_punishment, duplicate_tracking_punishment, as the
+        episode statistics hold them), the covered-target sum and the covered-target maximum.  Summed over environments
+        (maximum for the last field) an episode's rows equal its episode_stats() exactly."""
+        K, T = int(n_episodes), int(nsteps)
+        self._ensure_handle(config)
+        seeds = (C.c_uint64 * max(K, 1))(*[self._episode_seed(seed, self._episode + k) for k in range(max(K, 0))])
+        out = torch.empty((max(K, 0), self.n_envs, 6), dtype=torch.float64, device=self.device)
+        w, params = policy_weights(policy, self.state_dim, self.device)  # (params: kept alive over the call)
+        self._sync_weights(config)
+        mode, coop = self._mode(config, pmi)
+        with self._on_device():
+            _cabi.check(self._lib.uavsim_evaluate_policy(self._h, mode, coop, C.byref(w), int(bool(greedy)),
+                                                         C.c_uint64(policy_seed), C.c_uint64(first_counter),
+                                                         seeds if K > 0 else None, K, T,
+                                                         C.c_void_p(out.data_ptr()) if K > 0 else None, self._stream()),
+                        "uavsim_evaluate_policy")
+        self._episode += K
+        self._clear_traces()
+        return out
 
     def step_host(self, config, pmi, h_actions, h_obs=None, h_rew4=None, h_covered=None, chunks=4):
         """uavsim_step_host: host (ideally pinned) int32 actions [E,n] in, host obs/rew4/covered out."""

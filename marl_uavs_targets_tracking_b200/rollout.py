@@ -55,17 +55,16 @@ def policy_weights(policy, state_dim, device=None):
     return w, params
 
 
-def fused_policy_sample(policy, states, seed, counter, want_probs=False, out=None):
-    """One launch of libuavsim's fused policy kernel (`uavsim_policy_sample`, csrc/policy.cuh): softmax(fc2(relu(fc1(x))))
-    and one categorical draw per row, uniforms from Philox4x32-10 keyed (seed; row, counter).  `policy` is a PolicyNet
-    (or a DDP wrapper around one) on the device of `states` [B,12] float32; `out` = a contiguous int32 [B] tensor to write
-    the actions into (e.g. the environment's bound action buffer).  Returns (actions int32 [B], probs or None)."""
+def _fused_policy(name, policy, states, want_probs, out, key):
+    """One launch of the fused policy kernel through `name` (uavsim_policy_sample with key = (seed, counter), or
+    uavsim_policy_greedy with key = ())."""
     x = states if (states.dtype == torch.float32 and states.is_contiguous()) else states.float().contiguous()
     if x.data_ptr() % 16:  # the kernel reads rows with 16-byte loads: a view off a 16-byte boundary is copied
         x = x.clone()
     dev = x.device
     if dev.type != "cuda":
-        raise _cabi.UavSimError("fused_policy_sample needs CUDA tensors (no CPU fallback)")
+        raise _cabi.UavSimError("%s needs CUDA tensors (no CPU fallback)"
+                                % ("fused_policy_sample" if key else "fused_policy_greedy"))
     w, params = policy_weights(policy, x.shape[1], dev)
     B, A = x.shape[0], w.n_actions
     if out is not None:
@@ -74,12 +73,26 @@ def fused_policy_sample(policy, states, seed, counter, want_probs=False, out=Non
     probs = torch.empty(B, A, dtype=torch.float32, device=dev) if want_probs else None
     lib = _cabi.load()
     with torch.cuda.device(dev):
-        _cabi.check(lib.uavsim_policy_sample(C.c_void_p(x.data_ptr()), B, C.byref(w), C.c_uint64(seed), C.c_uint64(counter),
-                                             C.c_void_p(actions.data_ptr()),
-                                             C.c_void_p(probs.data_ptr()) if probs is not None else None,
-                                             dev.index or 0, C.c_void_p(torch.cuda.current_stream(dev).cuda_stream)),
-                    "uavsim_policy_sample")
+        _cabi.check(getattr(lib, name)(C.c_void_p(x.data_ptr()), B, C.byref(w), *(C.c_uint64(v) for v in key),
+                                       C.c_void_p(actions.data_ptr()),
+                                       C.c_void_p(probs.data_ptr()) if probs is not None else None,
+                                       dev.index or 0, C.c_void_p(torch.cuda.current_stream(dev).cuda_stream)), name)
     return actions, probs
+
+
+def fused_policy_sample(policy, states, seed, counter, want_probs=False, out=None):
+    """One launch of libuavsim's fused policy kernel (`uavsim_policy_sample`, csrc/policy.cuh): softmax(fc2(relu(fc1(x))))
+    and one categorical draw per row, uniforms from Philox4x32-10 keyed (seed; row, counter).  `policy` is a PolicyNet
+    (or a DDP wrapper around one) on the device of `states` [B,12] float32; `out` = a contiguous int32 [B] tensor to write
+    the actions into (e.g. the environment's bound action buffer).  Returns (actions int32 [B], probs or None)."""
+    return _fused_policy("uavsim_policy_sample", policy, states, want_probs, out, (seed, counter))
+
+
+def fused_policy_greedy(policy, states, want_probs=False, out=None):
+    """The greedy form of `fused_policy_sample` (`uavsim_policy_greedy`): the same forward, and per row the first index of
+    the largest probability the kernel computed -- torch.argmax of the returned probs.  Returns (actions int32 [B], probs
+    or None)."""
+    return _fused_policy("uavsim_policy_greedy", policy, states, want_probs, out, ())
 
 
 class BatchedActorCritic:
@@ -131,12 +144,17 @@ class BatchedActorCritic:
                 opt.load_state_dict(checkpoint["optimizer_state_dict"])
 
     @torch.no_grad()
-    def take_actions(self, states, out=None):
-        """states [B,12] float -> (actions [B] int32, probs [B,na] or None on the fused path)."""
+    def take_actions(self, states, out=None, greedy=False):
+        """states [B,12] float -> (actions [B] int32, probs [B,na] or None on the fused path).  greedy: the most probable
+        action (first index on ties) instead of a draw; it uses no random numbers, so the draw counter stays."""
         if self.fused:
+            if greedy:
+                return fused_policy_greedy(self.actor, states, out=out)
             self._calls += 1
             return fused_policy_sample(self.actor, states, self.seed, self._calls, out=out)
         probs = self.actor(states)
+        if greedy:
+            return probs.argmax(1).to(torch.int32), probs
         actions = torch.multinomial(probs, 1).squeeze(1)  # Categorical(probs).sample()
         return actions.to(torch.int32), probs
 
@@ -226,6 +244,60 @@ def operate_epoch_batched(config, env, agent, pmi, num_steps, keep_transitions=T
         transitions = None
     stats = reduce_episode_stats(env.episode_stats(), device=env.device)
     return transitions, episode_summary(stats, n)
+
+
+_ENV_STAT_KEYS = ("return", "target_tracking_return", "boundary_punishment_return", "duplicate_tracking_punishment_return",
+                  "average_covered_targets", "max_covered_targets")
+
+
+def evaluate_batched(config, env, agent, pmi, num_episodes, num_steps, greedy=False):
+    """The reference's evaluate phase (`--phase evaluate`, src/train.py evaluate) on every environment of `env`:
+    `num_episodes` episodes of `num_steps` steps, each from `env.reset(config)`, actions drawn by the agent's policy or,
+    with greedy, its most probable action.  Nothing is learned.
+
+    Returns (summaries, per_env).  summaries: one dict per episode, the scalars `operate_epoch_batched` reports
+    (`episode_summary` of the sums over all environments of all ranks).  per_env: dict of float64 [num_episodes, E]
+    tensors under the same keys -- return, the three term returns, average and max covered targets of every local
+    environment, normalised as `episode_summary` normalises (per agent-step, per step): the spread over seeds.
+
+    With the fused policy (agent.fused) all episodes are one library call, `env.evaluate_policy`
+    (uavsim_evaluate_policy); sampling advances agent._calls by num_episodes * num_steps, as take_actions would.  The
+    stock torch policy is driven step by step from Python and accumulates per environment in torch with the library's
+    fixed-point rule (`(v + 3.0f)` as int32 minus 0x40400000, summed as int64), so both paths give identical sums for
+    identical actions."""
+    E, n, dev = env.n_envs, env.n_uav, env.device
+    if getattr(agent, "fused", False):
+        rows = env.evaluate_policy(config, pmi, agent.actor, num_episodes, num_steps, greedy=greedy,
+                                   first_counter=agent._calls + 1, policy_seed=agent.seed)
+        if not greedy:
+            agent._calls += num_episodes * num_steps
+    else:
+        rows = torch.empty((num_episodes, E, 6), dtype=torch.float64, device=dev)
+        scale = torch.tensor([2.0 ** -22] * 4 + [1.0, 1.0], dtype=torch.float64, device=dev)
+        for k in range(num_episodes):
+            env.reset(config)
+            acc = torch.zeros((E, 6), dtype=torch.int64, device=dev)
+            for step in range(num_steps):
+                config["step"] = step + 1
+                a, _ = agent.take_actions(env._obs.view(E * n, 12), greedy=greedy)
+                _, rew4, covered = env.step_device(config, pmi, a.view(E, n))
+                acc[:, :4] += ((rew4 + 3.0).view(torch.int32) - 0x40400000).sum(2, dtype=torch.int64).T
+                acc[:, 4] += covered
+                acc[:, 5] = torch.maximum(acc[:, 5], covered.long())
+            rows[k] = acc.double() * scale
+    if num_steps > 0:
+        config["step"] = num_steps
+    sums = rows[:, :, :5].sum(1).tolist()
+    maxes = rows[:, :, 5].amax(1).tolist() if E else [0.0] * num_episodes
+    summaries = []
+    for s, mx in zip(sums, maxes):
+        stats = {"rewards": s[0], "target_tracking_reward": s[1], "boundary_punishment": s[2],
+                 "duplicate_tracking_punishment": s[3], "covered_sum": s[4], "covered_max": mx,
+                 "env_steps": float(E * num_steps)}
+        summaries.append(episode_summary(reduce_episode_stats(stats, device=dev), n))
+    norm = torch.tensor([max(num_steps * n, 1)] * 4 + [max(num_steps, 1), 1], dtype=torch.float64, device=dev)
+    per_env = rows / norm
+    return summaries, {k: per_env[:, :, q] for q, k in enumerate(_ENV_STAT_KEYS)}
 
 
 def train_batched(config, env, agent, pmi, num_episodes, num_steps, buffer=None, sample_size=None, on_episode=None):
