@@ -209,7 +209,8 @@ int uavsim_replay_sample(uavsim_replay_t *h, int64_t batch, double beta, const d
                          int64_t *o_indices, float *o_weights, int64_t *n_out, void *stream);
 
 /* update_priorities(indices, priorities) (src/train.py:134-136): sequential assignment, the last write to a
- * repeated index wins. */
+ * repeated index wins.  Precondition, not checked here (that would synchronise the stream): every priority is finite
+ * and non-negative (-0.0 counts as zero).  A NaN, infinite or negative priority makes later samples undefined. */
 int uavsim_replay_update_priorities(uavsim_replay_t *h, const int64_t *indices, const float *priorities,
                                     int64_t count, void *stream);
 

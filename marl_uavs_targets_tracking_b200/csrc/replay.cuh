@@ -34,12 +34,13 @@ struct uavsim_replay {
 };
 
 // ---- add ---------------------------------------------------------------------------------------
-// non-negative floats order like their bit patterns
+// As signed integers, non-negative floats order like their values and -0.0f (0x80000000, INT_MIN) ranks below +0.0f,
+// so `out` (cleared to +0.0f) ends at priorities.max() whichever zero fmaxf returns for a slot holding -0.0f.
 __global__ void replay_max_kernel(const float *__restrict__ pri, int64_t n, float *__restrict__ out) {
   float m = 0.f;
   for (int64_t i = blockIdx.x * (int64_t)blockDim.x + threadIdx.x; i < n; i += (int64_t)gridDim.x * blockDim.x) m = fmaxf(m, pri[i]);
   for (int o = 16; o; o >>= 1) m = fmaxf(m, __shfl_xor_sync(0xffffffffu, m, o));
-  if ((threadIdx.x & 31) == 0) atomicMax(reinterpret_cast<unsigned int *>(out), __float_as_uint(m));
+  if ((threadIdx.x & 31) == 0) atomicMax(reinterpret_cast<int *>(out), __float_as_int(m));
 }
 
 // rows [skip, count) of the batch go to ring slots (pos + k) % capacity; one thread per float of a row
@@ -121,7 +122,7 @@ __global__ void replay_norm_kernel(uavsim_replay R, int64_t n) {
   }
 }
 
-// one block: exclusive scan of the block sums in place (nblocks <= a few thousand)
+// one block: exclusive scan of the block sums in place (nblocks <= a few thousand); block_sums[nblocks] = the total
 __global__ void replay_scan_blocks_kernel(uavsim_replay R, int nblocks) {
   if (threadIdx.x == 0) {
     double run = 0;
@@ -130,24 +131,54 @@ __global__ void replay_scan_blocks_kernel(uavsim_replay R, int nblocks) {
   }
 }
 
-// inclusive fp64 scan inside each block of REPLAY_SCAN_ELEMS elements + the block's offset
+// Inclusive fp64 scan of each block of REPLAY_SCAN_ELEMS slots, placed between the block's offsets B_b = block_sums[b]
+// and B_{b+1} = fl(B_b + S_b) (replay_scan_blocks_kernel).  The in-block sums x_i (the thread's running sum on its offset
+// in the block) round differently from S_b and from the next thread's offset, so written as they are they could step
+// down at a thread, warp or block start and give a slot with p = 0 an interval an ulp wide.  Instead
+//   cdf_i = B_{b+1}                          from the block's last slot with p > 0 on,
+//   cdf_i = min(fl(B_b + M_i), B_{b+1})      before it, M_i = max of x_j over the block's slots j <= i with p_j > 0 (0 if none).
+// The maximum is exact in any order and fl(B_b + .) is monotone, so the CDF never steps down, and a slot with p = 0
+// repeats the value before it (B_b at a block's start, the previous block's last value): its interval is empty and the
+// search never returns it.  Every cdf_i stays within the rounding of the chains that made x_i, B_b and B_{b+1}.
 __global__ void replay_scan_kernel(uavsim_replay R, int64_t n) {
-  __shared__ double warp_tot[REPLAY_NT / 32];
+  __shared__ double warp_tot[REPLAY_NT / 32], warp_max[REPLAY_NT / 32];
+  __shared__ int warp_last[REPLAY_NT / 32];
   constexpr int PER = REPLAY_SCAN_ELEMS / REPLAY_NT;
   const int64_t base = (int64_t)blockIdx.x * REPLAY_SCAN_ELEMS + (int64_t)threadIdx.x * PER;
   double v[PER], run = 0;
+  unsigned pos = 0;  // bit k: slot base + k has p > 0
 #pragma unroll
-  for (int k = 0; k < PER; k++) { run += (base + k < n) ? (double)R.prob[base + k] : 0.0; v[k] = run; }
+  for (int k = 0; k < PER; k++) {
+    const float p = (base + k < n) ? R.prob[base + k] : 0.f;
+    run += (double)p;
+    v[k] = run;
+    if (p > 0.f) pos |= 1u << k;
+  }
   double inc = run;  // inclusive scan of the per-thread totals across the block
   const int lane = threadIdx.x & 31, wid = threadIdx.x >> 5;
   for (int o = 1; o < 32; o <<= 1) { const double u = __shfl_up_sync(0xffffffffu, inc, o); if (lane >= o) inc += u; }
   if (lane == 31) warp_tot[wid] = inc;
   __syncthreads();
-  double off = R.block_sums[blockIdx.x];
+  double off = 0;
   for (int w = 0; w < wid; w++) off += warp_tot[w];
   off += inc - run;
+  double m = 0;  // running maximum of x over the thread's slots with p > 0
 #pragma unroll
-  for (int k = 0; k < PER; k++) if (base + k < n) R.cdf[base + k] = off + v[k];
+  for (int k = 0; k < PER; k++) { if (pos >> k & 1) m = fmax(m, off + v[k]); v[k] = m; }
+  double mi = m;  // inclusive maximum over the warp's threads
+  for (int o = 1; o < 32; o <<= 1) { const double u = __shfl_up_sync(0xffffffffu, mi, o); if (lane >= o) mi = fmax(mi, u); }
+  double before = __shfl_up_sync(0xffffffffu, mi, 1);  // maximum over the block's earlier threads
+  if (lane == 0) before = 0;
+  const int wlast = __reduce_max_sync(0xffffffffu, pos ? (int)threadIdx.x * PER + 31 - __clz(pos) : -1);
+  if (lane == 31) warp_max[wid] = mi;
+  if (lane == 0) warp_last[wid] = wlast;
+  __syncthreads();
+  int last = -1;  // the block's last slot with p > 0
+  for (int w = 0; w < REPLAY_NT / 32; w++) { last = max(last, warp_last[w]); if (w < wid) before = fmax(before, warp_max[w]); }
+  const double b0 = R.block_sums[blockIdx.x], b1 = R.block_sums[blockIdx.x + 1];
+#pragma unroll
+  for (int k = 0; k < PER; k++)
+    if (base + k < n) R.cdf[base + k] = (int)threadIdx.x * PER + k >= last ? b1 : fmin(b0 + fmax(before, v[k]), b1);
 }
 
 // one thread per drawn sample: u -> index (searchsorted right on cdf / cdf[n-1]), gather the row, raw weight

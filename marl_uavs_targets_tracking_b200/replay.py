@@ -88,8 +88,15 @@ class PrioritizedReplayBuffer:
         pri = torch.as_tensor(batch_priorities).to(self.device, torch.float32).reshape(-1).contiguous()
         if idx.numel() != pri.numel():
             raise ValueError("indices and priorities differ in length")
-        if idx.numel() and (int(idx.min()) < 0 or int(idx.max()) >= self.capacity):
-            raise IndexError("replay index out of range")
+        if idx.numel():
+            # one host synchronisation for both checks, before anything is written.  A NaN, infinite or negative
+            # priority would give the next sample NaN or negative probabilities (the reference's numpy.random.choice
+            # raises there); -0.0 is a zero priority.
+            lo, hi, bad = torch.stack([idx.min(), idx.max(), (~torch.isfinite(pri) | (pri < 0)).any().long()]).tolist()
+            if lo < 0 or hi >= self.capacity:
+                raise IndexError("replay index out of range")
+            if bad:
+                raise ValueError("priorities must be finite and non-negative")
         _cabi.check(self._lib.uavsim_replay_update_priorities(self._h, _ptr(idx), _ptr(pri), idx.numel(), self._stream()),
                     "uavsim_replay_update_priorities")
 
